@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the MCEM VAE-NMF enhancement hot path (BASELINE.json metric: enhanced audio-seconds per second).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -18,6 +18,10 @@ Printed JSON line (rank 0): `value` times the device-resident path with CUDA eve
 inside the timed region; `cpu_baseline` is the CPU oracle port (the reference's algorithm, torch CPU ops) on the same
 workload in two host layouts - one utterance on all threads, and one single-threaded process per core (the reference's
 own layout) - with `value` the better of the two.
+
+`--dump-outputs DIR` writes what the timed path returned in its last timed step (rank 0's shard of the headline workload)
+as `DIR/<name>.npy`, see `dump_outputs`.  Inputs, weights and the sampler's seed depend only on the arguments, so two
+builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -60,7 +64,14 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the extra_configs blocks (BASELINE configs[2], configs[3])")
     ap.add_argument("--config3", action="store_true", help="run the configs[3] block at any GPU count (512 utterances x 16 chains per GPU)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the headline workload's outputs of the last timed step as DIR/<name>.npy (at most 64 MB)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
+    return args
 
 
 def measured_traffic(B, variant):
@@ -271,7 +282,29 @@ def synth_set(u0, count, seconds=SECONDS, threads=16):
     return [t[0] for t in trip], [t[1] for t in trip]
 
 
-def measure(variant, n_total, chains, steps, warmup, want_e2e, scaling, niter, sampler, rank, world, dev, label):
+DUMP_BYTES = 64 << 20
+DUMP_UTTERANCES = 128
+
+
+def dump_outputs(path, s_dev, n_dev, cost, utt_ids, T):
+    """Write what ``Enhancer.run_device`` returned: ``cost.npy`` the cost of every EM iteration and utterance ``[niter][B]``
+    (float64, complete), ``s_hat.npy`` / ``n_hat.npy`` the speech / noise estimates ``[k][T]`` (float32) of a fixed sample of
+    k <= 128 utterances (seed 0, in batch order) and ``utterance_ids.npy`` their global ids (float64): 64 MB at most."""
+    B = len(utt_ids)
+    cost_h = cost.to(torch.float64).cpu().numpy()
+    k = int(min(B, DUMP_UTTERANCES, max(1, (DUMP_BYTES - cost_h.nbytes) // (2 * 4 * T + 8))))
+    pick = np.sort(np.random.default_rng(0).choice(B, size=k, replace=False))
+    idx = torch.from_numpy(pick).to(s_dev.device)
+    out = dict(cost=cost_h,
+               s_hat=s_dev.view(B, T).index_select(0, idx).cpu().numpy(),
+               n_hat=n_dev.view(B, T).index_select(0, idx).cpu().numpy(),
+               utterance_ids=np.asarray(utt_ids, np.float64)[pick])
+    os.makedirs(path, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
+def measure(variant, n_total, chains, steps, warmup, want_e2e, scaling, niter, sampler, rank, world, dev, label, dump_dir=None):
     """One workload on this rank's shard; returns the JSON block (rank 0) or None.
 
     ``scaling`` "weak": ``n_total`` utterances PER RANK; "strong": ``n_total`` utterances split over the ranks with
@@ -341,6 +374,8 @@ def measure(variant, n_total, chains, steps, warmup, want_e2e, scaling, niter, s
     from dvae_b200 import tc
     tc.check_status(eng)
     value = n_all * SECONDS * steps / (ms_total * 1e-3)
+    if dump_dir and rank == 0:                                  # before the e2e block reuses the output buffers
+        dump_outputs(dump_dir, s_dev, n_dev, cost, utt_ids, T)
 
     # the path's only collective: per-utterance SI-SDR (packages/metrics.py:62-82, computed on the device) and final cost.
     # The first and last window of every utterance are left out: with center=False the overlap-add normalisation divides the
@@ -469,7 +504,8 @@ def run_b200(args):
         "BASELINE.json configs[%d] shape (%s, %d utterances per GPU)" % (2 if args.variant == "M2" else (3 if args.variant == "M2v3" else 1), args.variant, B)
     label = cfg_name + ": %s batch of %d synthetic 3 s 16 kHz utterances per GPU (all distinct), STFT 1024/256, NMF rank 10, %d EM iterations" % (
         args.variant, B, args.niter)
-    main = measure(args.variant, B, args.chains, args.steps, args.warmup, not args.no_e2e, "weak", args.niter, args.sampler, rank, world, dev, label)
+    main = measure(args.variant, B, args.chains, args.steps, args.warmup, not args.no_e2e, "weak", args.niter, args.sampler, rank, world, dev, label,
+                   dump_dir=args.dump_outputs)
 
     extra = []
     if headline and not args.no_extra:

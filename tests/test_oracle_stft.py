@@ -1,7 +1,5 @@
 """STFT / ISTFT restatement: cross-checks against torch.stft, a direct DFT and scipy.signal (librosa itself is not installable and
 the reference holds no vector at this boundary, see oracle/__init__.py)."""
-import os
-
 import numpy as np
 import pytest
 import torch
@@ -103,10 +101,15 @@ def test_errors():
         stft_np.istft(np.zeros((513, 4), np.complex64), fs=16000, wlen_sec=50.01e-3)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/data/subset"), reason="reference data only in the build container")
-def test_real_recording_vs_torch():
+def test_16bit_wav_vs_torch(tmp_path):
+    """A 16-bit PCM wav as the evaluation reads it (integer samples / 2^15), of a length that is not a whole number of hops:
+    the end-padding rule and the forward transform against torch.stft."""
     from scipy.io import wavfile
-    fs, w = wavfile.read("/root/reference/data/subset/processed/ntcd_timit/Noisy/Babble/-5/test/34M/sa1.wav")
+    from dvae_b200 import batch_io
+    x0, _, _ = synth.synth_utterance(6, 2.9)
+    batch_io.write_wav(str(tmp_path / "x.wav"), x0[:46397], 16000)
+    fs, w = wavfile.read(str(tmp_path / "x.wav"))
+    assert fs == 16000 and w.dtype == np.int16 and len(w) % 256 != 0
     x = w.astype(np.float64) / 32768.0
     X = stft_np.stft(x, **KW)
     xp = stft_np.end_pad(x, 16000, 64e-3, 0.25, 256)
