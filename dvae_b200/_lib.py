@@ -78,6 +78,7 @@ PROTOTYPES = {
                                     C.c_int64, C.c_int, c_ptr, c_ptr, c_ptr]),
     "dvae_wiener_from_a1": (C.c_int, [c_ptr, c_ptr, C.c_int, C.c_int64, C.c_int, C.c_int, c_ptr, c_ptr, C.c_int, c_ptr]),
     "dvae_energy_ratios": (C.c_int, [c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, C.c_int, c_ptr, c_ptr]),
+    "dvae_pcm16_f32": (C.c_int, [c_ptr, C.c_int64, c_ptr, c_ptr, c_ptr]),
     "dvae_resample_taps": (C.c_int, [C.c_int, c_ptr, C.c_int]),
     "dvae_resample_poly_f32": (C.c_int, [c_ptr, c_ptr, c_ptr, c_ptr, C.c_int, C.c_int, c_ptr, c_ptr, c_ptr, c_ptr, C.c_int64, c_ptr]),
     "dvae_stoi_workspace_bytes": (C.c_int64, [C.c_int, C.c_int64, C.c_int]),

@@ -62,9 +62,13 @@ def read_wav(path, channel=0):
 
 
 def write_wav(path, x, fs):
-    """16-bit PCM mono wav (``sf.write(path, x, fs)`` for float input: scale by 2^15, round, clip)."""
-    x = np.asarray(x, np.float64)
-    pcm = np.clip(np.rint(x * 32768.0), -32768, 32767).astype("<i2").tobytes()
+    """16-bit PCM mono wav (``sf.write(path, x, fs)`` for float input: scale by 2^15, round, clip).  An int16 array holds
+    the PCM samples already (``Enhancer.enhance(..., pcm16=True)``) and is written as it is."""
+    x = np.asarray(x)
+    if x.dtype == np.int16:
+        pcm = x.astype("<i2").tobytes()
+    else:
+        pcm = np.clip(np.rint(np.asarray(x, np.float64) * 32768.0), -32768, 32767).astype("<i2").tobytes()
     hdr = b"RIFF" + struct.pack("<I", 36 + len(pcm)) + b"WAVE" + b"fmt " + struct.pack("<IHHIIHH", 16, 1, 1, int(fs), int(fs) * 2, 2, 16) \
         + b"data" + struct.pack("<I", len(pcm))
     os.makedirs(os.path.dirname(os.path.abspath(path)), exist_ok=True)
@@ -84,8 +88,32 @@ def utterance_id(path: str) -> int:
     return zlib.crc32(path.encode("utf-8")) & 0x7FFFFFFF
 
 
+def _check_sublist(sublist, batch_size, fs, trim):
+    if int(batch_size) < 1:
+        raise ValueError("batch_size must be at least 1")
+    if fs <= 0 or (trim is not None and int(trim) < 0):
+        raise ValueError("fs must be positive and trim non-negative")
+    if any(len(ab) != 2 for ab in sublist):
+        raise ValueError("sublist must hold (proc_noisy_file_path, clean_file_path) pairs")
+
+
+def _require_files(paths):
+    for p in paths:
+        if not os.path.isfile(p):
+            raise FileNotFoundError("%s: no such file" % p)
+
+
+def _read_checked(path, fs, length=None):
+    x, f = read_wav(path)
+    if f != fs:
+        raise ValueError("%s: sampling rate %d, expected %d" % (path, f, fs))
+    if length is not None and len(x) != length:
+        raise ValueError("%s: %d samples, expected %d" % (path, len(x), length))
+    return np.asarray(x, np.float32)
+
+
 def process_sublist(sublist, enhancer, processed_wav_dir, output_data_dir, batch_size=512, max_frames=None, labels=None,
-                    io_threads=8, fs=16000, utt_ids=None):
+                    io_threads=8, fs=16000, utt_ids=None, score=False):
     """Batched replacement of ``process_sublist`` / ``process_utt`` (scripts/evaluate_ntcd_M1.py:81-214).
 
     ``sublist``: ``(proc_noisy_file_path, clean_file_path)`` pairs as the reference builds them.  Files whose
@@ -95,28 +123,48 @@ def process_sublist(sublist, enhancer, processed_wav_dir, output_data_dir, batch
     (default: ``utterance_id``, a hash of the path), so every utterance gets its own draws whatever ``batch_size`` and
     sharding are - the reference draws fresh numbers per utterance too.  File I/O overlaps the GPU work: the next batch is read and
     the previous one written by ``io_threads`` workers while the current one is enhanced.  Returns the list of written stems.
+
+    ``score=True`` also reads the clean file ``processed_wav_dir + clean_file_path`` of every pair, scores each estimate on
+    the device while its batch is enhanced (``Enhancer.enhance(..., ref_list=..., pcm16=True)``: the score of exactly the
+    16-bit samples written) and returns ``(written_stems, scores [n][2][5])`` (``metrics.SCORE_KEYS``; row 0 the estimate,
+    row 1 the noisy input).  The files are the same bytes as without ``score``; ``score_sublist`` on them gives the same
+    numbers.
     """
+    if score:
+        _check_sublist(sublist, batch_size, fs, None)
     utt_ids = utt_ids or utterance_id
     todo = [(a, b) for a, b in sublist if not os.path.exists(output_stem(output_data_dir, a) + "_s_est.wav")]
-    written = []
+    if score:
+        _require_files([processed_wav_dir + p for ab in todo for p in ab])
+    written, scores = [], []
     with ThreadPoolExecutor(max(1, io_threads)) as pool:
         pending = None                                               # futures of the previous batch's wav writes
-        submit_reads = lambda part: [pool.submit(read_wav, processed_wav_dir + ab[0]) for ab in part]
+
+        def submit_reads(part):
+            return [(pool.submit(_read_checked, processed_wav_dir + ab[0], fs),
+                     pool.submit(_read_checked, processed_wav_dir + ab[1], fs) if score else None) for ab in part]
+
         reads = submit_reads(todo[:batch_size])
         for lo in range(0, len(todo), batch_size):
             part = todo[lo:lo + batch_size]
-            sigs = [f.result() for f in reads]
+            xs = [f.result() for f, _ in reads]
+            cs = [g.result() for _, g in reads] if score else None
             reads = submit_reads(todo[lo + batch_size:lo + 2 * batch_size])      # read ahead: the next batch loads while this one runs
-            for (x, f), ab in zip(sigs, part):
-                if f != fs:
-                    raise ValueError("%s: sampling rate %d, expected %d" % (ab[0], f, fs))
-            xs = [np.asarray(x, np.float32) for x, _ in sigs]
+            if score:
+                for x, c, ab in zip(xs, cs, part):
+                    if len(c) != len(x):
+                        raise ValueError("%s: %d samples, the noisy file has %d" % (processed_wav_dir + ab[1], len(c), len(x)))
             caps = [max_frames(*ab) for ab in part] if max_frames else None
             if caps is not None and any(c is None for c in caps):
                 big = np.iinfo(np.int64).max
                 caps = [big if c is None else c for c in caps]
             ys = [labels(*ab) for ab in part] if labels else None
-            s_hat, n_hat, _ = enhancer.enhance(xs, y_list=ys, max_frames_list=caps, utt_ids=[utt_ids(ab[0]) for ab in part])
+            ids = [utt_ids(ab[0]) for ab in part]
+            if score:
+                s_hat, n_hat, _, sc = enhancer.enhance(xs, y_list=ys, max_frames_list=caps, utt_ids=ids, ref_list=cs, pcm16=True)
+                scores.append(sc)
+            else:
+                s_hat, n_hat, _ = enhancer.enhance(xs, y_list=ys, max_frames_list=caps, utt_ids=ids)
             if pending:
                 for fut in pending:
                     fut.result()
@@ -130,4 +178,48 @@ def process_sublist(sublist, enhancer, processed_wav_dir, output_data_dir, batch
         if pending:
             for fut in pending:
                 fut.result()
-    return written
+    if not score:
+        return written
+    return written, (np.concatenate(scores) if scores else np.zeros((0, 2, 5)))
+
+
+def score_sublist(sublist, processed_wav_dir, output_data_dir, device=0, batch_size=512, io_threads=8, fs=16000, trim=None):
+    """Batched replacement of the scoring loop of the reference's ``scripts/run_metrics.py``: SI-SDR, SI-SIR, SI-SAR, STOI and
+    ESTOI (``metrics.SCORE_KEYS``) of every pair's ``*_s_est.wav`` on the GPU, in ragged batches of ``batch_size``.
+
+    For each ``(proc_noisy_file_path, clean_file_path)`` pair it reads the estimate ``output_stem(output_data_dir, noisy) +
+    "_s_est.wav"``, the noisy file ``processed_wav_dir + noisy`` and the clean file ``processed_wav_dir + clean``; the next
+    batch is read by ``io_threads`` workers while the current one is scored (``metrics.score_batch``, trim as there).
+    Returns ``(stems, scores [n][2][5])`` float64, row 0 the estimate and row 1 the noisy input; the rows feed
+    ``metrics.compute_stats``.  A missing file raises ``FileNotFoundError`` before any device work.
+    """
+    _check_sublist(sublist, batch_size, fs, trim)
+    stems = [output_stem(output_data_dir, a) for a, _ in sublist]
+    triples = [(st + "_s_est.wav", processed_wav_dir + a, processed_wav_dir + b) for st, (a, b) in zip(stems, sublist)]
+    _require_files([p for t in triples for p in t])
+    import torch
+    from .engine import _require_cuda
+    from .packages import metrics
+    dev = _require_cuda(device)
+    out = []
+
+    def read_triple(t):
+        x = _read_checked(t[1], fs)
+        return _read_checked(t[0], fs, len(x)), x, _read_checked(t[2], fs, len(x))
+
+    with ThreadPoolExecutor(max(1, io_threads)) as pool, torch.cuda.device(dev):
+        reads = [pool.submit(read_triple, t) for t in triples[:batch_size]]
+        for lo in range(0, len(triples), batch_size):
+            sigs = [f.result() for f in reads]
+            reads = [pool.submit(read_triple, t) for t in triples[lo + batch_size:lo + 2 * batch_size]]
+            lens = np.array([len(x) for _, x, _ in sigs], np.int32)
+            off = np.zeros(len(sigs) + 1, np.int64)
+            np.cumsum((lens.astype(np.int64) + 1) // 2 * 2, out=off[1:])            # even offsets, as Enhancer.enhance
+            flat = np.zeros((3, int(off[-1])), np.float32)
+            for u, trip in enumerate(sigs):
+                for k in range(3):
+                    flat[k, off[u]:off[u] + lens[u]] = trip[k]
+            est, x, s = (torch.from_numpy(flat[k]).to(dev) for k in range(3))
+            out.append(metrics.score_batch(est, x, s, torch.from_numpy(off[:-1].copy()).to(dev), torch.from_numpy(lens).to(dev), fs,
+                                           trim=trim).cpu().numpy())
+    return stems, (np.concatenate(out) if out else np.zeros((0, 2, 5)))

@@ -630,8 +630,8 @@ class Enhancer:
             self._pinned[name] = t
         return t[:n]
 
-    def _pin_out(self, n):
-        """A pinned float32 result buffer leased to the caller: ``(tensor, ndarray)``.
+    def _pin_out(self, n, dtype=torch.float32):
+        """A pinned result buffer of ``dtype`` leased to the caller: ``(tensor, ndarray)``.
 
         Results are returned as views of pinned memory (no extra host copy).  Ownership is explicit: every lease gets a
         FRESH ndarray object over the pinned storage, the result views handed out keep that object alive through their
@@ -640,8 +640,8 @@ class Enhancer:
         reference counts are inspected.
         """
         import weakref
-        k = next((i for i, t in enumerate(self._out_free) if t.numel() >= n), None)
-        t = self._out_free.pop(k) if k is not None else torch.empty(n, dtype=torch.float32).pin_memory()
+        k = next((i for i, t in enumerate(self._out_free) if t.numel() >= n and t.dtype == dtype), None)
+        t = self._out_free.pop(k) if k is not None else torch.empty(n, dtype=dtype).pin_memory()
         a = t.numpy()                                              # new ndarray object per lease
         free = self._out_free
 
@@ -691,8 +691,10 @@ class Enhancer:
         return s_dev, n_dev, cost
 
     @_on_device
-    def enhance(self, x_list, y_list=None, utt_ids=None, max_frames_list=None, draws=None, return_device=False, s_list=None):
-        """Enhance a list of 1-D float32 host signals.  Returns ``(s_hat_list, n_hat_list, cost [B][niter])``.
+    def enhance(self, x_list, y_list=None, utt_ids=None, max_frames_list=None, draws=None, return_device=False, s_list=None,
+                ref_list=None, pcm16=False):
+        """Enhance a list of 1-D float32 host signals.  Returns ``(s_hat_list, n_hat_list, cost [B][niter])``, and the scores
+        ``[B][2][5]`` as a fourth element when ``ref_list`` is given.
 
         ``y_list``: per-utterance label arrays ``(y_dim, N_u)`` as the reference passes them (M2 variants).
         ``max_frames_list``: optional per-utterance frame caps (the reference truncates to the video length).
@@ -700,6 +702,12 @@ class Enhancer:
         of the clean speech (``clean_speech_VAD``, scripts/evaluate_ntcd_M2.py), computed on the device.
         ``utt_ids``: global utterance ids = Philox counter word 0; callers that enhance several batches must pass distinct
         ids per utterance (``batch_io.process_sublist`` does), or every batch replays the same random draws.
+        ``ref_list``: clean signals, one per utterance and of its length, to score against on the device
+        (``metrics.score_batch`` with its default trim, ``SCORE_KEYS`` order): row ``[u][0]`` scores the speech estimate
+        after 16-bit PCM quantisation, i.e. exactly the samples ``batch_io.write_wav`` stores, row ``[u][1]`` the input.
+        It may be the same list as ``s_list``; it then is copied to the device once.
+        ``pcm16=True`` returns both estimates as int16 PCM (``write_wav``'s quantisation, done on the device), which halves
+        their device-to-host bytes.  Neither option changes the estimates.
         ``return_device=True`` returns device tensors that alias the engine's output buffers: they are valid until the
         next call on this Enhancer (clone them to keep them).
         """
@@ -711,6 +719,8 @@ class Enhancer:
         nfr = np.array([num_frames(int(t), self.n_fft, self.hop, self.fs) for t in lens], np.int64)
         if np.any(nfr < 1):
             raise ValueError("utterance shorter than one STFT frame")
+        if ref_list is not None and (len(ref_list) != B or any(len(a) != t for a, t in zip(ref_list, lens))):
+            raise ValueError("ref_list needs one clean signal per utterance, of the utterance's length")
         if max_frames_list is not None:
             nfr = np.minimum(nfr, np.asarray(max_frames_list, np.int64))
         off = np.zeros(B + 1, np.int64)
@@ -724,14 +734,15 @@ class Enhancer:
         x_off = torch.from_numpy(off[:-1].copy()).to(dev)
         x_len = torch.from_numpy(lens).to(dev)
         batch = RaggedBatch(nfr, dev, utt_ids)
-        y = None
+        y = s_dev_in = None
         if self.weights.y_dim and y_list is None and s_list is not None:
             if self.weights.y_dim != 1 or len(s_list) != B or any(len(a) != t for a, t in zip(s_list, lens)):
                 raise ValueError("device VAD labels need one clean signal per utterance and a model with one label input")
             from .packages.processing.target import vad_batch
             hs_in = self._pin("s_in", total, torch.float32)
             self._stage(hs_in.numpy(), s_list, off, lens)
-            y = vad_batch(hs_in.to(dev, non_blocking=True), x_off, x_len, batch, self.n_fft, self.hop).view(batch.NT, 1)
+            s_dev_in = hs_in.to(dev, non_blocking=True)
+            y = vad_batch(s_dev_in, x_off, x_len, batch, self.n_fft, self.hop).view(batch.NT, 1)
         elif self.weights.y_dim:
             if y_list is None:
                 raise ValueError("this model needs labels y")
@@ -739,22 +750,46 @@ class Enhancer:
             if yc.shape != (batch.NT, self.weights.y_dim):
                 raise ValueError("labels do not cover the frames")
             y = torch.from_numpy(np.ascontiguousarray(yc)).to(dev)
+        ref_dev = None
+        if ref_list is not None:
+            if ref_list is s_list and s_dev_in is not None:
+                ref_dev = s_dev_in
+            else:
+                hr = self._pin("ref", total, torch.float32)
+                self._stage(hr.numpy(), ref_list, off, lens)
+                ref_dev = hr.to(dev, non_blocking=True)
         self._h2d_done = torch.cuda.Event()
         self._h2d_done.record()
         s_dev, n_dev, cost = self.run_device(x_dev, x_off, x_len, batch, y, total, int(lens.max()), draws)
-        self.h2d_bytes = total * 4 + (0 if y is None else y.numel() * 4)
-        self.d2h_bytes = 2 * total * 4 + cost.numel() * 8
+        self.h2d_bytes = total * 4 + (0 if y is None else y.numel() * 4) + (0 if ref_dev is None else total * 4)
+        scores = None
+        if ref_list is not None or pcm16:
+            from .packages import metrics
+            s_pcm = eng._get("s_pcm", (total,), torch.int16) if pcm16 else None
+            n_pcm = eng._get("n_pcm", (total,), torch.int16) if pcm16 else None
+            s_q = eng._get("s_q", (total,)) if ref_list is not None else None
+            metrics.pcm16(s_dev, s_pcm, s_q)
+            if pcm16:
+                metrics.pcm16(n_dev, n_pcm)
+                s_dev, n_dev = s_pcm, n_pcm
+            if ref_list is not None:
+                scores = metrics.score_batch(s_q, x_dev, ref_dev, x_off, x_len, self.fs, out=eng._get("scores", (B, 2, 5), torch.float64))
+        esize = 2 if pcm16 else 4
+        self.d2h_bytes = 2 * total * esize + cost.numel() * 8 + (0 if scores is None else scores.numel() * 8)
         from . import tc
         if return_device:
             tc.check_status(eng)                               # synchronises
-            return s_dev, n_dev, cost
-        hs, s_np = self._pin_out(total)
-        hn, n_np = self._pin_out(total)
+            return (s_dev, n_dev, cost) if scores is None else (s_dev, n_dev, cost, scores)
+        hs, s_np = self._pin_out(total, s_dev.dtype)
+        hn, n_np = self._pin_out(total, n_dev.dtype)
         hs[:total].copy_(s_dev, non_blocking=True)
         hn[:total].copy_(n_dev, non_blocking=True)
         cost_h = cost.t().contiguous().cpu()                   # synchronises the stream
+        scores_h = None if scores is None else scores.cpu().numpy()
         torch.cuda.current_stream().synchronize()
         tc.check_status(eng)
         s_list = [s_np[off[u]:off[u] + lens[u]] for u in range(B)]      # views of pinned memory, see _pin_out
         n_list = [n_np[off[u]:off[u] + lens[u]] for u in range(B)]
-        return s_list, n_list, cost_h.numpy()
+        if scores_h is None:
+            return s_list, n_list, cost_h.numpy()
+        return s_list, n_list, cost_h.numpy(), scores_h

@@ -4,7 +4,9 @@ Same names, arguments and return values as the reference for the per-utterance f
 numpy arrays out); the arithmetic runs in ``dvae_energy_ratios`` (six inner products in double, closed forms for the
 energies) instead of forming ``s_target``, ``e_noise`` and ``e_art``.  ``energy_ratios_batch`` is the batched entry the
 enhancement path uses: device tensors in the layout of ``Enhancer.run_device``, nothing leaves the GPU but 24 bytes per
-utterance.  CUDA only: without the library or a device the calls raise ``DvaeError``.
+utterance.  ``score_batch`` puts SI-SDR / SI-SIR / SI-SAR and STOI / ESTOI of a batch together (the scoring loop of the
+reference's ``scripts/run_metrics.py``), ``pcm16`` quantises device signals as ``batch_io.write_wav`` does.  CUDA only: without
+the library or a device the calls raise ``DvaeError``.
 """
 from __future__ import annotations
 
@@ -152,6 +154,64 @@ def stoi(x, y, fs_sig, extended=False, device=None):
         warnings.warn("Not enough STFT frames to compute intermediate intelligibility measure after removing silent "
                       "frames. Returning 1e-5. Please check you wav files", RuntimeWarning)
     return float(r[1 if extended else 0])
+
+
+# --------------------------------------------------------------------------------------------- 16-bit PCM and batched scoring
+SCORE_KEYS = ("si_sdr", "si_sir", "si_sar", "stoi", "estoi")
+
+
+def pcm16(x, pcm=None, xq=None):
+    """16-bit PCM quantisation of the float32 CUDA tensor ``x`` exactly as ``batch_io.write_wav`` does it
+    (``clip(rint(x * 32768), -32768, 32767)``, round half to even; NaN maps to 0): writes the int16 samples into ``pcm`` and
+    ``q / 32768`` (what ``read_wav`` returns for the written file) into ``xq``.  Either may be None, not both; given ones
+    must be contiguous tensors of ``x``'s size.  Enqueued on the current stream."""
+    if not x.is_cuda or x.dtype != torch.float32 or not x.is_contiguous():
+        raise ValueError("x must be a contiguous float32 CUDA tensor")
+    for t, dt in ((pcm, torch.int16), (xq, torch.float32)):
+        if t is not None and (t.dtype != dt or t.numel() != x.numel() or not t.is_contiguous() or t.device != x.device):
+            raise ValueError("pcm / xq must be contiguous %s tensors of x's size on x's device" % dt)
+    with torch.cuda.device(x.device):
+        _lib.call("dvae_pcm16_f32", _p(x), x.numel(), _p(pcm), _p(xq), _stream())
+    return pcm, xq
+
+
+def score_batch(est, x, s, off, lens, fs, trim=None, out=None):
+    """SI-SDR, SI-SIR, SI-SAR, STOI and ESTOI (``SCORE_KEYS``) of a ragged batch, for the estimate and for the mixture.
+
+    ``est`` (speech estimate), ``x`` (noisy mixture), ``s`` (clean speech): 1-D float32 CUDA tensors in the layout of
+    ``Enhancer.run_device`` (utterance u is ``[off[u], off[u] + lens[u])``), sampled at ``fs`` Hz.  Returns a float64 CUDA
+    tensor ``[B][2][5]`` (written into ``out`` when given): row ``[u][0]`` scores ``est``, row ``[u][1]`` scores ``x``, so
+    ``[u][0] - [u][1]`` is the improvement.  The noise reference of SI-SIR / SI-SAR is ``n = x - s`` (exact for additive
+    mixtures).
+
+    Every metric is computed on ``[off + trim, off + lens - trim)``: the reference's ``run_metrics.py`` drops 50 ms at both
+    ends before scoring (default ``trim = round(0.05 fs)``, 800 samples at 16 kHz).  Whether it trims before ESTOI as well is
+    not verified; here all five metrics see the same trimmed signal.  A row is NaN when ``lens <= 2 trim``; otherwise STOI's
+    own rules apply (1e-5 below 30 frames, NaN where undefined).  Enqueued on the current stream; nothing synchronises.
+    """
+    if not all(t.is_cuda for t in (est, x, s, off, lens)):
+        raise _lib.DvaeError("score_batch needs CUDA tensors")
+    if not all(t.dtype == torch.float32 and t.dim() == 1 and t.shape == x.shape for t in (est, s, x)):
+        raise ValueError("est, x and s must be 1-D float32 tensors of the same length")
+    trim = int(round(0.05 * fs)) if trim is None else int(trim)
+    if trim < 0 or fs <= 0:
+        raise ValueError("fs must be positive and trim non-negative")
+    B, dev = int(off.numel()), x.device
+    if out is None:
+        out = torch.empty((B, 2, 5), dtype=torch.float64, device=dev)
+    elif out.shape != (B, 2, 5) or out.dtype != torch.float64 or not out.is_contiguous() or out.device != dev:
+        raise ValueError("out must be a contiguous float64 [B][2][5] tensor on the signals' device")
+    with torch.cuda.device(dev):
+        est, x, s = est.contiguous(), x.contiguous(), s.contiguous()
+        n = torch.sub(x, s)
+        lens = lens.to(torch.int64)
+        t_off = off.to(torch.int64) + trim
+        t_len = torch.clamp_min(lens - 2 * trim, 0).to(torch.int32)
+        for k, sig in enumerate((est, x)):
+            out[:, k, :3] = energy_ratios_batch(sig, s, n, t_off, t_len)
+            out[:, k, 3:] = stoi_batch(s, sig, t_off, t_len, int(fs))
+        out.masked_fill_((lens <= 2 * trim).view(B, 1, 1), float("nan"))
+    return out
 
 
 def si_sdr_components(s_hat, s, n):

@@ -267,6 +267,12 @@ int dvae_nmf_w_from_frame_stats(const float* A1, const float* A2, const float* P
 int dvae_energy_ratios(const float* s_hat, const float* s, const float* n, const int64_t* off, const int32_t* len, int B,
                        double* out, void* stream);
 
+/* ---- 16-bit PCM quantisation (batch_io.write_wav: np.clip(np.rint(x * 32768), -32768, 32767).astype("<i2")) ----
+ * Over the flat buffer x[0..n): q = clamp(rint(x * 32768), -32768, 32767), round half to even, +-Inf saturating, NaN -> 0.
+ * pcm[i] = q (the samples of the wav file) and xq[i] = q / 32768 (what read_wav returns for it, exact in FP32); either
+ * output may be null, not both.  16-byte aligned x / xq and 8-byte aligned pcm take the vectorised path. */
+int dvae_pcm16_f32(const float* x, int64_t n, int16_t* pcm /* nullable */, float* xq /* nullable */, void* stream);
+
 /* ---- STOI / ESTOI on the device (pystoi.stoi, called by scripts/run_metrics.py) ----
  * Ragged batch of (clean x, processed y) pairs: utterance u occupies [off[u], off[u] + len[u]) of x and y, sampled at fs_sig.
  * dvae_resample_taps [host only, no GPU needed]: Octave's anti-aliasing filter that pystoi hands to scipy's resample_poly
