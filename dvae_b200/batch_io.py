@@ -113,7 +113,7 @@ def _read_checked(path, fs, length=None):
 
 
 def process_sublist(sublist, enhancer, processed_wav_dir, output_data_dir, batch_size=512, max_frames=None, labels=None,
-                    io_threads=8, fs=16000, utt_ids=None, score=False):
+                    io_threads=8, fs=16000, utt_ids=None, score=False, score_at=()):
     """Batched replacement of ``process_sublist`` / ``process_utt`` (scripts/evaluate_ntcd_M1.py:81-214).
 
     ``sublist``: ``(proc_noisy_file_path, clean_file_path)`` pairs as the reference builds them.  Files whose
@@ -129,14 +129,24 @@ def process_sublist(sublist, enhancer, processed_wav_dir, output_data_dir, batch
     16-bit samples written) and returns ``(written_stems, scores [n][2][5])`` (``metrics.SCORE_KEYS``; row 0 the estimate,
     row 1 the noisy input).  The files are the same bytes as without ``score``; ``score_sublist`` on them gives the same
     numbers.
+
+    ``score_at`` (with ``score=True``): EM iteration counts as ``Enhancer.enhance(..., score_at=...)`` takes them; the call
+    then returns ``(written_stems, scores, trace [n][len(score_at)][5])``, where ``trace[u][k]`` is the estimate's score row
+    that a run with ``niter = score_at[k]`` would give, all from this one run.  The files do not change.
     """
+    score_at = tuple(score_at)
+    if score_at and not score:
+        raise ValueError("score_at needs score=True")
     if score:
         _check_sublist(sublist, batch_size, fs, None)
+    if score_at:
+        from .engine import check_checkpoints
+        score_at = check_checkpoints(score_at, enhancer.cfg.niter)
     utt_ids = utt_ids or utterance_id
     todo = [(a, b) for a, b in sublist if not os.path.exists(output_stem(output_data_dir, a) + "_s_est.wav")]
     if score:
         _require_files([processed_wav_dir + p for ab in todo for p in ab])
-    written, scores = [], []
+    written, scores, traces = [], [], []
     with ThreadPoolExecutor(max(1, io_threads)) as pool:
         pending = None                                               # futures of the previous batch's wav writes
 
@@ -161,8 +171,10 @@ def process_sublist(sublist, enhancer, processed_wav_dir, output_data_dir, batch
             ys = [labels(*ab) for ab in part] if labels else None
             ids = [utt_ids(ab[0]) for ab in part]
             if score:
-                s_hat, n_hat, _, sc = enhancer.enhance(xs, y_list=ys, max_frames_list=caps, utt_ids=ids, ref_list=cs, pcm16=True)
+                s_hat, n_hat, _, sc, *tr = enhancer.enhance(xs, y_list=ys, max_frames_list=caps, utt_ids=ids, ref_list=cs, pcm16=True,
+                                                            score_at=score_at)
                 scores.append(sc)
+                traces += tr
             else:
                 s_hat, n_hat, _ = enhancer.enhance(xs, y_list=ys, max_frames_list=caps, utt_ids=ids)
             if pending:
@@ -180,7 +192,10 @@ def process_sublist(sublist, enhancer, processed_wav_dir, output_data_dir, batch
                 fut.result()
     if not score:
         return written
-    return written, (np.concatenate(scores) if scores else np.zeros((0, 2, 5)))
+    scores = np.concatenate(scores) if scores else np.zeros((0, 2, 5))
+    if not score_at:
+        return written, scores
+    return written, scores, (np.concatenate(traces) if traces else np.zeros((0, len(score_at), 5)))
 
 
 def score_sublist(sublist, processed_wav_dir, output_data_dir, device=0, batch_size=512, io_threads=8, fs=16000, trim=None):

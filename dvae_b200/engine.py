@@ -595,16 +595,69 @@ class McemEngine:
         self.WFs, self.WFn, self.R_wf = WFs, WFn, R
 
     @_on_device
-    def run(self, draws: Optional[InjectedDraws] = None):
+    def run(self, draws: Optional[InjectedDraws] = None, checkpoints: Sequence[int] = (), on_checkpoint=None):
         """``EM.run`` (mcem.py:156-179): niter x (E-step, M-step, cost), then the Wiener estimates.
 
         Returns the device cost matrix ``[niter][B]`` (float64); nothing synchronises with the host.
+
+        ``checkpoints``: EM iteration counts (``check_checkpoints``) at which ``on_checkpoint(n)`` is called while ``S_hat`` /
+        ``N_hat`` hold the estimates that a run with ``niter = n`` returns, bit for bit: the MH draws are keyed by the global
+        MH iteration, not by the call, so the final filter run on the side after M-step ``n`` draws what that run's own
+        filter draws.  The side run's state is restored afterwards, so the main run does not change.  For ``n == niter`` the
+        call follows the run's own filter.  Not with injected ``draws``: they are indexed by call and would be consumed out
+        of order.
         """
+        cps = check_checkpoints(checkpoints, self.cfg.niter)
+        if cps and draws is not None:
+            raise ValueError("checkpoints need the engine's own random numbers, not injected draws")
         for it in range(self.cfg.niter):
             self.e_step(draws)
             self.m_step(it)
+            if it + 1 in cps and it + 1 < self.cfg.niter:
+                self._side_filter(it + 1, on_checkpoint)
         self.wiener(draws)
+        if on_checkpoint is not None and self.cfg.niter in cps:
+            on_checkpoint(self.cfg.niter)
         return self.cost
+
+    def _side_filter(self, n, on_checkpoint):
+        """The final filter from the current state, ``on_checkpoint(n)``, then the state as it was before the filter.  The
+        filter moves the chains (``Z``), the acceptance counts and the MH counters, and points the E-step's emission
+        attributes elsewhere; Z and n_accept are snapshotted with device copies, the rest are host attributes.  The buffers
+        it overwrites (filter samples, masks, spectra, the FP32 ``Vs`` scratch) are rewritten by the next E-step before any
+        read.  Device time goes to the stage "trace" alone."""
+        Z0 = self._get("Z_trace", self.Z.shape)
+        acc0 = self._get("n_accept_trace", self.n_accept.shape, torch.int32)
+        Z0.copy_(self.Z)
+        acc0.copy_(self.n_accept)
+        names = ("mh_calls", "mh_iter0", "mh_rows", "_Vs", "vst_R", "_last_Zs", "VsT", "vs_idx")
+        saved = {k: getattr(self, k) for k in names if hasattr(self, k)}
+        with self.stage("trace"):
+            timing, self.timing = self.timing, False
+            try:
+                self.wiener()
+                if on_checkpoint is not None:
+                    on_checkpoint(n)
+            finally:
+                self.timing = timing
+        self.Z.copy_(Z0)
+        self.n_accept.copy_(acc0)
+        for k, v in saved.items():
+            setattr(self, k, v)
+
+
+def check_checkpoints(checkpoints: Sequence[int], niter: int) -> tuple:
+    """``checkpoints`` as a tuple of ints after checking they are sorted, unique integers in ``[1, niter]``; ``ValueError``
+    otherwise.  No device work."""
+    cps = tuple(checkpoints)
+    if not all(isinstance(n, (int, np.integer)) and not isinstance(n, bool) for n in cps):
+        raise ValueError("checkpoints must be integers, got %r" % (cps,))
+    cps = tuple(int(n) for n in cps)
+    if any(b <= a for a, b in zip(cps, cps[1:])):
+        raise ValueError("checkpoints must be sorted and unique, got %r" % (cps,))
+    if cps and (cps[0] < 1 or cps[-1] > niter):
+        raise ValueError("checkpoints must lie in [1, niter=%d], got %r" % (niter, cps))
+    return cps
 
 
 # --------------------------------------------------------------------------------------------- end-to-end helper
@@ -673,16 +726,17 @@ class Enhancer:
             f.result()
 
     @_on_device
-    def run_device(self, x_dev, x_off, x_len, batch, y, total, max_len, draws=None):
+    def run_device(self, x_dev, x_off, x_len, batch, y, total, max_len, draws=None, checkpoints=(), on_checkpoint=None):
         """The whole path on device-resident inputs: STFT -> MCEM -> Wiener -> ISTFT.  Nothing touches the host.
 
         ``x_dev``: concatenated float32 signals; ``x_off`` / ``x_len``: per-utterance offsets / lengths (device);
-        returns ``(s_hat, n_hat)`` in the layout of ``x_dev`` and the cost matrix ``[niter][B]``.
+        returns ``(s_hat, n_hat)`` in the layout of ``x_dev`` and the cost matrix ``[niter][B]``.  ``checkpoints`` /
+        ``on_checkpoint`` go to ``McemEngine.run`` (see ``checkpoint_scorer``).
         """
         eng = self.engine
         X, P = stft_batch(x_dev, x_off, x_len, batch, self.n_fft, self.hop)
         eng.init_parameters(X, P, batch, y, draws)
-        cost = eng.run(draws)
+        cost = eng.run(draws, checkpoints, on_checkpoint)
         s_dev = istft_batch(eng.S_hat, batch, x_off, x_len, total, max_len, self.n_fft, self.hop,
                             out=eng._get("s_out", (total,)))
         n_dev = istft_batch(eng.N_hat, batch, x_off, x_len, total, max_len, self.n_fft, self.hop,
@@ -690,11 +744,27 @@ class Enhancer:
         eng.kernel_launches += 4          # stft, power-free init kernels are counted there; 2 istft + stft + vb
         return s_dev, n_dev, cost
 
+    def checkpoint_scorer(self, ref, x_off, x_len, batch, total, max_len, rows):
+        """An ``on_checkpoint`` for ``run_device`` that scores each checkpoint's speech estimate the way ``enhance`` scores
+        ``scores[:, 0]``: ISTFT of ``S_hat`` as in ``run_device``, 16-bit PCM quantisation, then ``metrics.score_row``
+        against ``ref`` (``metrics.score_reference``) into ``rows[n]``, a float64 ``[B][5]`` view.  Nothing synchronises."""
+        from .packages import metrics
+        eng = self.engine
+
+        def score(n):
+            est = istft_batch(eng.S_hat, batch, x_off, x_len, total, max_len, self.n_fft, self.hop,
+                              out=eng._get("s_out", (total,)))
+            s_q = eng._get("s_q", (total,))
+            metrics.pcm16(est, None, s_q)
+            metrics.score_row(s_q, ref, rows[n])
+        return score
+
     @_on_device
     def enhance(self, x_list, y_list=None, utt_ids=None, max_frames_list=None, draws=None, return_device=False, s_list=None,
-                ref_list=None, pcm16=False):
+                ref_list=None, pcm16=False, score_at=()):
         """Enhance a list of 1-D float32 host signals.  Returns ``(s_hat_list, n_hat_list, cost [B][niter])``, and the scores
-        ``[B][2][5]`` as a fourth element when ``ref_list`` is given.
+        ``[B][2][5]`` as a fourth element when ``ref_list`` is given, and the trace ``[B][len(score_at)][5]`` as a fifth when
+        ``score_at`` is.
 
         ``y_list``: per-utterance label arrays ``(y_dim, N_u)`` as the reference passes them (M2 variants).
         ``max_frames_list``: optional per-utterance frame caps (the reference truncates to the video length).
@@ -708,6 +778,11 @@ class Enhancer:
         It may be the same list as ``s_list``; it then is copied to the device once.
         ``pcm16=True`` returns both estimates as int16 PCM (``write_wav``'s quantisation, done on the device), which halves
         their device-to-host bytes.  Neither option changes the estimates.
+        ``score_at``: sorted, unique EM iteration counts in ``[1, niter]`` (needs ``ref_list``, not ``draws``).  Entry
+        ``[u][k]`` of the trace (float64, ``SCORE_KEYS`` columns) is the score row ``[u][0]`` that this call with
+        ``niter = score_at[k]`` would return, bit for bit; the input's row ``[u][1]`` does not change with ``niter``.  The
+        whole curve comes from this one run (``McemEngine.run(checkpoints=...)``), and the estimates, cost and scores are
+        those of the call without ``score_at``.
         ``return_device=True`` returns device tensors that alias the engine's output buffers: they are valid until the
         next call on this Enhancer (clone them to keep them).
         """
@@ -721,6 +796,9 @@ class Enhancer:
             raise ValueError("utterance shorter than one STFT frame")
         if ref_list is not None and (len(ref_list) != B or any(len(a) != t for a, t in zip(ref_list, lens))):
             raise ValueError("ref_list needs one clean signal per utterance, of the utterance's length")
+        score_at = check_checkpoints(score_at, eng.cfg.niter)
+        if score_at and (ref_list is None or draws is not None):
+            raise ValueError("score_at needs ref_list and the engine's own random numbers (no injected draws)")
         if max_frames_list is not None:
             nfr = np.minimum(nfr, np.asarray(max_frames_list, np.int64))
         off = np.zeros(B + 1, np.int64)
@@ -760,7 +838,14 @@ class Enhancer:
                 ref_dev = hr.to(dev, non_blocking=True)
         self._h2d_done = torch.cuda.Event()
         self._h2d_done.record()
-        s_dev, n_dev, cost = self.run_device(x_dev, x_off, x_len, batch, y, total, int(lens.max()), draws)
+        trace = on_checkpoint = None
+        if score_at:
+            from .packages import metrics
+            trace = eng._get("trace", (B, len(score_at), 5), torch.float64)
+            on_checkpoint = self.checkpoint_scorer(metrics.score_reference(x_dev, ref_dev, x_off, x_len, self.fs), x_off, x_len,
+                                                   batch, total, int(lens.max()), {n: trace[:, k] for k, n in enumerate(score_at)})
+        side = tuple(n for n in score_at if n < eng.cfg.niter)    # niter itself is the run's own filter, scored below
+        s_dev, n_dev, cost = self.run_device(x_dev, x_off, x_len, batch, y, total, int(lens.max()), draws, side, on_checkpoint)
         self.h2d_bytes = total * 4 + (0 if y is None else y.numel() * 4) + (0 if ref_dev is None else total * 4)
         scores = None
         if ref_list is not None or pcm16:
@@ -774,22 +859,23 @@ class Enhancer:
                 s_dev, n_dev = s_pcm, n_pcm
             if ref_list is not None:
                 scores = metrics.score_batch(s_q, x_dev, ref_dev, x_off, x_len, self.fs, out=eng._get("scores", (B, 2, 5), torch.float64))
+            if score_at and score_at[-1] == eng.cfg.niter:
+                trace[:, -1].copy_(scores[:, 0])
         esize = 2 if pcm16 else 4
-        self.d2h_bytes = 2 * total * esize + cost.numel() * 8 + (0 if scores is None else scores.numel() * 8)
+        self.d2h_bytes = 2 * total * esize + cost.numel() * 8 + sum(0 if t is None else t.numel() * 8 for t in (scores, trace))
+        extra = () if scores is None else (scores,) if trace is None else (scores, trace)
         from . import tc
         if return_device:
             tc.check_status(eng)                               # synchronises
-            return (s_dev, n_dev, cost) if scores is None else (s_dev, n_dev, cost, scores)
+            return (s_dev, n_dev, cost) + extra
         hs, s_np = self._pin_out(total, s_dev.dtype)
         hn, n_np = self._pin_out(total, n_dev.dtype)
         hs[:total].copy_(s_dev, non_blocking=True)
         hn[:total].copy_(n_dev, non_blocking=True)
         cost_h = cost.t().contiguous().cpu()                   # synchronises the stream
-        scores_h = None if scores is None else scores.cpu().numpy()
+        extra = tuple(t.cpu().numpy() for t in extra)
         torch.cuda.current_stream().synchronize()
         tc.check_status(eng)
         s_list = [s_np[off[u]:off[u] + lens[u]] for u in range(B)]      # views of pinned memory, see _pin_out
         n_list = [n_np[off[u]:off[u] + lens[u]] for u in range(B)]
-        if scores_h is None:
-            return s_list, n_list, cost_h.numpy()
-        return s_list, n_list, cost_h.numpy(), scores_h
+        return (s_list, n_list, cost_h.numpy()) + extra

@@ -5,10 +5,13 @@ numpy arrays out); the arithmetic runs in ``dvae_energy_ratios`` (six inner prod
 energies) instead of forming ``s_target``, ``e_noise`` and ``e_art``.  ``energy_ratios_batch`` is the batched entry the
 enhancement path uses: device tensors in the layout of ``Enhancer.run_device``, nothing leaves the GPU but 24 bytes per
 utterance.  ``score_batch`` puts SI-SDR / SI-SIR / SI-SAR and STOI / ESTOI of a batch together (the scoring loop of the
-reference's ``scripts/run_metrics.py``), ``pcm16`` quantises device signals as ``batch_io.write_wav`` does.  CUDA only: without
+reference's ``scripts/run_metrics.py``; ``score_reference`` + ``score_row`` are its two halves, for scoring several estimates
+against one reference), ``pcm16`` quantises device signals as ``batch_io.write_wav`` does.  CUDA only: without
 the library or a device the calls raise ``DvaeError``.
 """
 from __future__ import annotations
+
+from typing import NamedTuple
 
 import numpy as np
 import torch
@@ -189,28 +192,61 @@ def score_batch(est, x, s, off, lens, fs, trim=None, out=None):
     not verified; here all five metrics see the same trimmed signal.  A row is NaN when ``lens <= 2 trim``; otherwise STOI's
     own rules apply (1e-5 below 30 frames, NaN where undefined).  Enqueued on the current stream; nothing synchronises.
     """
-    if not all(t.is_cuda for t in (est, x, s, off, lens)):
+    if not est.is_cuda:
         raise _lib.DvaeError("score_batch needs CUDA tensors")
-    if not all(t.dtype == torch.float32 and t.dim() == 1 and t.shape == x.shape for t in (est, s, x)):
+    if est.dtype != torch.float32 or est.dim() != 1 or est.shape != x.shape:
         raise ValueError("est, x and s must be 1-D float32 tensors of the same length")
+    ref = score_reference(x, s, off, lens, fs, trim)
+    B = int(off.numel())
+    if out is None:
+        out = torch.empty((B, 2, 5), dtype=torch.float64, device=x.device)
+    elif out.shape != (B, 2, 5) or out.dtype != torch.float64 or not out.is_contiguous() or out.device != x.device:
+        raise ValueError("out must be a contiguous float64 [B][2][5] tensor on the signals' device")
+    for k, sig in enumerate((est, x)):
+        score_row(sig, ref, out[:, k])
+    return out
+
+
+class ScoreReference(NamedTuple):
+    """What every scored row of a batch shares (``score_reference``): clean speech ``s``, noise ``n = x - s``, the trimmed
+    layout ``t_off`` / ``t_len``, the rows too short to score (``short``, bool ``[B]``) and the sample rate."""
+    s: torch.Tensor
+    n: torch.Tensor
+    t_off: torch.Tensor
+    t_len: torch.Tensor
+    short: torch.Tensor
+    fs: int
+
+
+def score_reference(x, s, off, lens, fs, trim=None):
+    """The clean side of ``score_batch`` for mixture ``x`` and clean speech ``s`` (arguments as there), computed once so that
+    any number of estimates can be scored against it with ``score_row``.  Enqueued on the current stream."""
+    if not all(t.is_cuda for t in (x, s, off, lens)):
+        raise _lib.DvaeError("score_batch needs CUDA tensors")
+    if not all(t.dtype == torch.float32 and t.dim() == 1 and t.shape == x.shape for t in (s, x)):
+        raise ValueError("x and s must be 1-D float32 tensors of the same length")
     trim = int(round(0.05 * fs)) if trim is None else int(trim)
     if trim < 0 or fs <= 0:
         raise ValueError("fs must be positive and trim non-negative")
-    B, dev = int(off.numel()), x.device
-    if out is None:
-        out = torch.empty((B, 2, 5), dtype=torch.float64, device=dev)
-    elif out.shape != (B, 2, 5) or out.dtype != torch.float64 or not out.is_contiguous() or out.device != dev:
-        raise ValueError("out must be a contiguous float64 [B][2][5] tensor on the signals' device")
-    with torch.cuda.device(dev):
-        est, x, s = est.contiguous(), x.contiguous(), s.contiguous()
-        n = torch.sub(x, s)
+    with torch.cuda.device(x.device):
+        s = s.contiguous()
+        n = torch.sub(x.contiguous(), s)
         lens = lens.to(torch.int64)
-        t_off = off.to(torch.int64) + trim
-        t_len = torch.clamp_min(lens - 2 * trim, 0).to(torch.int32)
-        for k, sig in enumerate((est, x)):
-            out[:, k, :3] = energy_ratios_batch(sig, s, n, t_off, t_len)
-            out[:, k, 3:] = stoi_batch(s, sig, t_off, t_len, int(fs))
-        out.masked_fill_((lens <= 2 * trim).view(B, 1, 1), float("nan"))
+        return ScoreReference(s, n, off.to(torch.int64) + trim, torch.clamp_min(lens - 2 * trim, 0).to(torch.int32),
+                              lens <= 2 * trim, int(fs))
+
+
+def score_row(est, ref, out):
+    """One row of ``score_batch``: the five ``SCORE_KEYS`` of the 1-D float32 CUDA signal ``est`` against ``ref``
+    (``score_reference``), written into the float64 ``[B][5]`` view ``out``; NaN where the utterance is too short for the
+    trim.  Enqueued on the current stream; nothing synchronises."""
+    if not est.is_cuda or est.dtype != torch.float32 or est.dim() != 1 or est.shape != ref.s.shape:
+        raise ValueError("est must be a 1-D float32 CUDA tensor of the reference's length")
+    with torch.cuda.device(est.device):
+        est = est.contiguous()
+        out[:, :3] = energy_ratios_batch(est, ref.s, ref.n, ref.t_off, ref.t_len)
+        out[:, 3:] = stoi_batch(ref.s, est, ref.t_off, ref.t_len, ref.fs)
+        out.masked_fill_(ref.short.view(-1, 1), float("nan"))
     return out
 
 
