@@ -452,6 +452,27 @@ extern "C" int dvae_tc_decoder_exponent_bound(const DvaeMlp* dec, int L, int y_d
     return 0;
 }
 
+extern "C" int64_t dvae_tc_image_bias_offset(const DvaeMlp* dec, int L, int y_dim) {
+    Dims d;
+    if (check_dims(dec, L, y_dim, "dvae_tc_image_bias_offset", &d)) return -1;
+    return d.off_bias + 4 * (d.n_hidden == 2 ? HID : 0);           // the layer-3 bias follows the hidden-2 bias (pack_decoder_kernel)
+}
+
+// The samplers' hidden activation (hidden_rows_bf_part) over every BF16 input: table[x] = tanh.approx.bf16x2 of pattern x
+__global__ void tanh_bf16_table_kernel(uint16_t* __restrict__ out) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;      // one pair of patterns per thread
+    if (i >= 32768u) return;
+    const uint32_t y = tanh_bf16x2((2u * i) | ((2u * i + 1u) << 16));
+    out[2 * i] = (uint16_t)(y & 0xffffu);
+    out[2 * i + 1] = (uint16_t)(y >> 16);
+}
+
+extern "C" int dvae_tc_tanh_bf16_table(uint16_t* out, void* stream) {
+    DVAE_REQUIRE(out != nullptr, "dvae_tc_tanh_bf16_table: null pointer");
+    tanh_bf16_table_kernel<<<128, 256, 0, (cudaStream_t)stream>>>(out);
+    return check_launch("tanh_bf16_table_kernel");
+}
+
 extern "C" int64_t dvae_tc_packed_pv_bytes(int64_t chains) {
     if (chains <= 0) return 0;
     return ((chains + TM - 1) / TM) * (int64_t)NQ * TM * 16;

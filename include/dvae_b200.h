@@ -198,6 +198,13 @@ int dvae_tc_row_scale(const DvaeMlp* dec, const void* image, int L, int y_dim, c
 int dvae_tc_pack_pv(const DvaeMlp* dec, const void* image, int L, int y_dim, const float* P, const float* Vb,
                     const float* kscale, int64_t NT, int n_chains, int F, int ld, void* dst, void* stream);
 int dvae_tc_decoder_exponent_bound(const DvaeMlp* dec, int L, int y_dim, float* bound_host, void* stream);
+/* Byte offset inside the decoder image of the FP32 layer-3 bias in the log2 domain (b3 * log2 e, the per-bin scale the P / Vb
+ * stream is packed with), or -1. */
+int64_t dvae_tc_image_bias_offset(const DvaeMlp* dec, int L, int y_dim);
+/* The samplers' hidden-layer activation (tanh.approx.bf16x2 on the BF16-rounded pre-activation) as a table over every input:
+ * out[x] (65536 BF16 bit patterns, device memory) = the activation of the BF16 number with bit pattern x.  For parity tests:
+ * the instruction is not the correctly rounded tanh. */
+int dvae_tc_tanh_bf16_table(uint16_t* out, void* stream);
 int64_t dvae_vst_bytes(int64_t chains, int n_keep);
 int dvae_mh_chain_tc2(const DvaeMlp* dec, const void* image, const void* PVpk, const float* kscale, const float* g, const float* y, int y_dim,
                       const float* ybias /* nullable: [NT][128] */, const int32_t* frame_utt, const int32_t* frame_idx, float* Z,
