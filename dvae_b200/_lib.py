@@ -17,7 +17,7 @@ MAX_LAYERS = 6
 MAX_L = 64
 MAX_K = 16
 ACT_NONE, ACT_TANH, ACT_EXP = 0, 1, 2
-ABI_VERSION = 2
+ABI_VERSION = 3
 STATUS_TIMEOUT, STATUS_NONFINITE = 1, 2
 
 c_f32p = C.c_void_p      # device pointers are passed as integers
@@ -31,7 +31,15 @@ class DvaeMlp(C.Structure):
 
 class DvaeRng(C.Structure):
     _fields_ = [("seed", C.c_uint64), ("iter0", C.c_uint32), ("reserved", C.c_uint32),
-                ("eps", C.c_void_p), ("u", C.c_void_p)]
+                ("eps", C.c_void_p), ("u", C.c_void_p), ("iter0_frame", C.c_void_p)]
+
+
+PERMUTE_MAX_JOBS = 16
+
+
+class DvaePermuteJob(C.Structure):
+    _fields_ = [("src", C.c_void_p), ("dst", C.c_void_p), ("map", C.c_void_p), ("n_rows", C.c_int64), ("row_bytes", C.c_int64),
+                ("n_rep", C.c_int64), ("pitch", C.c_int64)]
 
 
 # name -> (restype, argtypes); mirrors include/dvae_b200.h one to one
@@ -106,6 +114,8 @@ PROTOTYPES = {
     "dvae_nmf_w_from_partials": (C.c_int, [c_ptr, c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, C.c_int, c_ptr, c_ptr]),
     "dvae_vst_unpack": (C.c_int, [C.POINTER(DvaeMlp), c_ptr, C.c_int, C.c_int, c_ptr, c_ptr, C.c_int, C.c_int64, C.c_int, c_ptr, c_ptr]),
     "dvae_vst_pack": (C.c_int, [C.POINTER(DvaeMlp), c_ptr, C.c_int, C.c_int, c_ptr, C.c_int, C.c_int64, C.c_int, c_ptr, c_ptr, c_ptr]),
+    "dvae_em_stop_check": (C.c_int, [c_ptr, C.c_int, C.c_int, C.c_int, C.c_int, C.c_double, c_ptr, c_ptr]),
+    "dvae_permute_rows": (C.c_int, [C.POINTER(DvaePermuteJob), C.c_int, c_ptr]),
     "dvae_nmf_init": (C.c_int, [C.c_uint64, c_ptr, c_ptr, C.c_int, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_float,
                                 c_ptr, c_ptr, c_ptr, c_ptr]),
 }

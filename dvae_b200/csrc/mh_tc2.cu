@@ -62,6 +62,7 @@ struct Mh2Params {
     // slot 1 + r = the proposal of kept iteration r.  vs_idx[chain][32]: byte r = slot holding kept sample r.
     uint4* VsT;
     uint8_t* vs_idx;
+    const uint32_t* iter0_frame;  // per-frame iter0 [frames] (mh2_kernel<.., .., true>) or null
 };
 
 
@@ -129,7 +130,9 @@ __device__ __forceinline__ uint4 ld_pv(const uint4* p, uint64_t pol) {
     return v;
 }
 
-template <int L, int POLY>
+// PER_FRAME: the Philox iteration base comes from p.iter0_frame (a separate instantiation, so that the kernel without it keeps
+// its instruction stream)
+template <int L, int POLY, bool PER_FRAME>
 __global__ void __launch_bounds__(MH2_THREADS, 1) mh2_kernel(Mh2Params p) {
     extern __shared__ unsigned char smem_raw[];
     __shared__ uint64_t bars[6];                       // layer 1/2 ready, chunk ready x3, buffer free x2
@@ -141,6 +144,7 @@ __global__ void __launch_bounds__(MH2_THREADS, 1) mh2_kernel(Mh2Params p) {
     unsigned char* A = base + ((d.image_bytes + 1023) & ~1023);
     float2* red2 = reinterpret_cast<float2*>(A + A_BYTES);       // [2][128] {partial l(z'), partial prior term} of each column half
     float* u_sh = reinterpret_cast<float*>(red2 + 2 * TM);       // [128] accept uniform of the next proposal (written by half 0)
+    uint32_t* it0_sh = reinterpret_cast<uint32_t*>(u_sh + TM);    // [128] the row's Philox iteration base, with iter0_frame only
     const uint32_t bar12 = smem_u32(&bars[0]);
     const uint32_t bar3_0 = smem_u32(&bars[1]), bar3_1 = smem_u32(&bars[2]);
     const uint32_t barf_0 = smem_u32(&bars[3]);
@@ -221,6 +225,8 @@ __global__ void __launch_bounds__(MH2_THREADS, 1) mh2_kernel(Mh2Params p) {
         float y0 = 0.f, y1 = 0.f, y2 = 0.f, ll_cur = 0.f, u_cur = 0.5f, prior_h = 0.f;
         uint32_t n_acc = 0, state_slot = 0;
         int prop = 0;                                      // index of the next proposal to draw
+        // the frame's own iter0 (DvaeRng.iter0_frame) waits in shared memory: one more register would make the kernel spill
+        if constexpr (PER_FRAME) it0_sh[row] = valid ? __ldg(p.iter0_frame + fr) : 0u;
 #pragma unroll
         for (int l = 0; l < LH; ++l) { zh[l] = valid ? p.Z[row_g * L + h * LH + l] : 0.f; zph[l] = 0.f; }
 #pragma unroll
@@ -247,7 +253,7 @@ __global__ void __launch_bounds__(MH2_THREADS, 1) mh2_kernel(Mh2Params p) {
                     if (owner) u_sh[row] = __ldg(p.u + (int64_t)prop * p.rows + row_g);
                 }
             } else {
-                const uint32_t iter = p.iter0 + (uint32_t)prop;
+                const uint32_t iter = (PER_FRAME ? it0_sh[row] : p.iter0) + (uint32_t)prop;
                 constexpr int HALF = (LH / 4 + 1) / 2;              // blocks in part 0
 #pragma unroll
                 for (int l = 0; l < LH / 4; ++l) {
@@ -507,6 +513,7 @@ extern "C" int dvae_mh_chain_tc2(const DvaeMlp* dec, const void* image, const vo
     DVAE_REQUIRE(!ybias || (reinterpret_cast<uintptr_t>(ybias) & 15) == 0, "dvae_mh_chain_tc2: ybias must be 16-byte aligned");
     DVAE_REQUIRE(NT >= 0 && n_chains >= 1 && n_chains < 4096 && n_burn >= 0 && n_keep >= 1 && var_rw > 0.f, "dvae_mh_chain_tc2: bad sizes");
     DVAE_REQUIRE((rng->eps == nullptr) == (rng->u == nullptr), "dvae_mh_chain_tc2: eps and u must be injected together");
+    DVAE_REQUIRE(!(rng->eps && rng->iter0_frame), "dvae_mh_chain_tc2: iter0_frame applies to Philox draws only");
     DVAE_REQUIRE(rng->eps || (frame_utt && frame_idx), "dvae_mh_chain_tc2: Philox mode needs frame_utt / frame_idx");
     DVAE_REQUIRE((reinterpret_cast<uintptr_t>(Zs) & 15) == 0 && (reinterpret_cast<uintptr_t>(rng->eps) & 15) == 0,
                  "dvae_mh_chain_tc2: Zs and eps must be 16-byte aligned");
@@ -520,20 +527,27 @@ extern "C" int dvae_mh_chain_tc2(const DvaeMlp* dec, const void* image, const vo
     p.eps = rng->eps; p.u = rng->u;
     p.frame_gid = frame_utt; p.frame_idx = frame_idx;
     p.keys = philox_keys((uint32_t)(rng->seed & 0xffffffffu), (uint32_t)(rng->seed >> 32)); p.iter0 = rng->iter0;
+    p.iter0_frame = rng->iter0_frame;
     p.n_accept = n_accept; p.a_trace = a_trace; p.n_burn = n_burn; p.n_keep = n_keep;
     p.sd = sqrtf(var_rw);
     p.status = status;
     p.VsT = (uint4*)VsT; p.vs_idx = vs_idx;
-    const size_t smem = smem_bytes(p.d) + (size_t)TM * 20;       // + red2 [2][128] float2 and u_sh [128] behind the activation operand
+    // + red2 [2][128] float2, u_sh [128] and, with iter0_frame, it0_sh [128] behind the activation operand
+    const size_t smem = smem_bytes(p.d) + (size_t)TM * (rng->iter0_frame ? 24 : 20);
     DVAE_REQUIRE(smem <= 227 * 1024, "dvae_mh_chain_tc2: shared memory budget exceeded");
     const int64_t n_tiles = (p.rows + TM - 1) / TM;
     const int grid = (int)(n_tiles < 148 ? n_tiles : 148);
     cudaStream_t st = (cudaStream_t)stream;
     const int poly = (flags & DVAE_TC_POLY_EX2_ALL) ? 2 : ((flags & DVAE_TC_POLY_EX2) ? 1 : 0);
-#define MH2_LAUNCH(LL, PP)                                                                                   \
-    do {                                                                                                     \
-        cudaFuncSetAttribute(mh2_kernel<LL, PP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);    \
-        mh2_kernel<LL, PP><<<grid, MH2_THREADS, smem, st>>>(p);                                              \
+#define MH2_LAUNCH2(LL, PP, PF)                                                                                  \
+    do {                                                                                                         \
+        cudaFuncSetAttribute(mh2_kernel<LL, PP, PF>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);    \
+        mh2_kernel<LL, PP, PF><<<grid, MH2_THREADS, smem, st>>>(p);                                              \
+    } while (0)
+#define MH2_LAUNCH(LL, PP)                          \
+    do {                                            \
+        if (p.iter0_frame) MH2_LAUNCH2(LL, PP, true); \
+        else MH2_LAUNCH2(LL, PP, false);            \
     } while (0)
     if (L == 16 && poly == 2) MH2_LAUNCH(16, 2);
     else if (L == 16 && poly == 1) MH2_LAUNCH(16, 1);
@@ -542,5 +556,6 @@ extern "C" int dvae_mh_chain_tc2(const DvaeMlp* dec, const void* image, const vo
     else if (poly == 1) MH2_LAUNCH(32, 1);
     else MH2_LAUNCH(32, 0);
 #undef MH2_LAUNCH
+#undef MH2_LAUNCH2
     return check_launch("mh2_kernel");
 }

@@ -205,6 +205,7 @@ struct MhArgs {
     int64_t chains;
     int L, C, n_tiles, n_burn, n_keep;
     uint32_t seed_lo, seed_hi, iter0;
+    const uint32_t* iter0_frame;  // nullable [NT]: per-frame iter0
     float sd;
 };
 
@@ -252,7 +253,7 @@ __global__ void __launch_bounds__(128) mh_step_kernel(MhArgs a, int it) {
             const int64_t fr = m / a.C;
             const uint32_t c = (uint32_t)(m - fr * a.C);
             mh_draws(a.seed_lo, a.seed_hi, (uint32_t)a.frame_utt[fr], (uint32_t)a.frame_idx[fr] | (c << 20),
-                     a.iter0 + (uint32_t)nxt, L, eps, u);
+                     (a.iter0_frame ? a.iter0_frame[fr] : a.iter0) + (uint32_t)nxt, L, eps, u);
         }
         for (int l = 0; l < L; ++l) zp[l] = __fadd_rn(z[l], __fmul_rn(a.sd, eps[l]));
         a.u_next[m] = u;
@@ -263,8 +264,8 @@ __global__ void copy_rows_kernel(const float* __restrict__ src, float* __restric
     for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) dst[i] = src[i];
 }
 
-__global__ void rng_dump_kernel(uint32_t seed_lo, uint32_t seed_hi, uint32_t iter0, const int32_t* __restrict__ frame_utt,
-                                const int32_t* __restrict__ frame_idx, int64_t chains, int C, int L, int n_iter,
+__global__ void rng_dump_kernel(uint32_t seed_lo, uint32_t seed_hi, uint32_t iter0, const uint32_t* __restrict__ iter0_frame,
+                                const int32_t* __restrict__ frame_utt, const int32_t* __restrict__ frame_idx, int64_t chains, int C, int L, int n_iter,
                                 float* __restrict__ eps_out, float* __restrict__ u_out) {
     const int64_t total = chains * n_iter;
     for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
@@ -274,7 +275,8 @@ __global__ void rng_dump_kernel(uint32_t seed_lo, uint32_t seed_hi, uint32_t ite
         const uint32_t c = (uint32_t)(m - fr * C);
         float eps[DVAE_MAX_L];
         float u;
-        mh_draws(seed_lo, seed_hi, (uint32_t)frame_utt[fr], (uint32_t)frame_idx[fr] | (c << 20), iter0 + (uint32_t)it, L, eps, u);
+        mh_draws(seed_lo, seed_hi, (uint32_t)frame_utt[fr], (uint32_t)frame_idx[fr] | (c << 20),
+                 (iter0_frame ? iter0_frame[fr] : iter0) + (uint32_t)it, L, eps, u);
         for (int l = 0; l < L; ++l) eps_out[i * L + l] = eps[l];
         u_out[i] = u;
     }
@@ -284,7 +286,7 @@ __global__ void rng_dump_kernel(uint32_t seed_lo, uint32_t seed_hi, uint32_t ite
 // Same counters and the same arithmetic as mh_draws, so the numbers are bit-identical to rng_dump_kernel.
 // blockIdx.y = MH iteration, blockIdx.x covers chains * nb blocks: no 64-bit division on the index path.
 __global__ void __launch_bounds__(256) rng_dump4_kernel(uint32_t seed_lo, uint32_t seed_hi, uint32_t iter0,
-                                                        const int32_t* __restrict__ frame_utt, const int32_t* __restrict__ frame_idx,
+                                                        const uint32_t* __restrict__ iter0_frame, const int32_t* __restrict__ frame_utt, const int32_t* __restrict__ frame_idx,
                                                         uint32_t chains, uint32_t C, uint32_t nb_shift, float4* __restrict__ eps_out,
                                                         float* __restrict__ u_out) {
     const uint32_t it = blockIdx.y;
@@ -295,7 +297,7 @@ __global__ void __launch_bounds__(256) rng_dump4_kernel(uint32_t seed_lo, uint32
         const uint32_t fr = (C == 1) ? m : m / C;
         const uint32_t c = (C == 1) ? 0u : m - fr * C;
         const uint32_t utt = (uint32_t)__ldg(frame_utt + fr), fc = (uint32_t)__ldg(frame_idx + fr) | (c << 20);
-        const Philox4 r = philox4x32_10(utt, fc, iter0 + it, b, seed_lo, seed_hi);
+        const Philox4 r = philox4x32_10(utt, fc, (iter0_frame ? __ldg(iter0_frame + fr) : iter0) + it, b, seed_lo, seed_hi);
         float4 o;
         box_muller(r.x, r.y, o.x, o.y);
         box_muller(r.z, r.w, o.z, o.w);
@@ -371,6 +373,7 @@ extern "C" int dvae_mh_chain_f32(const DvaeMlp* dec, const float* P, const float
     DVAE_REQUIRE(n_burn >= 0 && n_keep >= 1, "dvae_mh_chain_f32: bad schedule");
     DVAE_REQUIRE(var_rw > 0.f, "dvae_mh_chain_f32: var_rw must be positive");
     DVAE_REQUIRE((rng->eps == nullptr) == (rng->u == nullptr), "dvae_mh_chain_f32: eps and u must be injected together");
+    DVAE_REQUIRE(!(rng->eps && rng->iter0_frame), "dvae_mh_chain_f32: iter0_frame applies to Philox draws only");
     DVAE_REQUIRE(rng->eps || (frame_utt && frame_idx), "dvae_mh_chain_f32: Philox mode needs frame_utt/frame_idx");
     if (NT == 0) return 0;
     cudaStream_t st = (cudaStream_t)stream;
@@ -389,6 +392,7 @@ extern "C" int dvae_mh_chain_f32(const DvaeMlp* dec, const float* P, const float
     a.n_accept = n_accept; a.a_trace = a_trace; a.chains = chains; a.L = L; a.C = n_chains; a.n_tiles = n_tiles;
     a.n_burn = n_burn; a.n_keep = n_keep;
     a.seed_lo = (uint32_t)(rng->seed & 0xffffffffu); a.seed_hi = (uint32_t)(rng->seed >> 32); a.iter0 = rng->iter0;
+    a.iter0_frame = rng->iter0_frame;
     a.sd = sqrtf(var_rw);
 
     LoglikArgs ll{P, Vb, g, partial, ld, n_chains, n_tiles};
@@ -420,13 +424,13 @@ extern "C" int dvae_rng_dump(const DvaeRng* rng, const int32_t* frame_utt, const
         const uint32_t per_it = chains << nb_shift;
         const uint32_t bx = (per_it + 255) / 256;
         rng_dump4_kernel<<<dim3(bx < 4096 ? bx : 4096, n_iter), 256, 0, (cudaStream_t)stream>>>(
-            (uint32_t)(rng->seed & 0xffffffffu), (uint32_t)(rng->seed >> 32), rng->iter0, frame_utt, frame_idx, chains,
+            (uint32_t)(rng->seed & 0xffffffffu), (uint32_t)(rng->seed >> 32), rng->iter0, rng->iter0_frame, frame_utt, frame_idx, chains,
             (uint32_t)n_chains, nb_shift, reinterpret_cast<float4*>(eps), u);
         return check_launch("rng_dump4_kernel");
     }
     const int grid = (int)((total + 127) / 128 < 148 * 16 ? (total + 127) / 128 : 148 * 16);
     rng_dump_kernel<<<grid, 128, 0, (cudaStream_t)stream>>>((uint32_t)(rng->seed & 0xffffffffu), (uint32_t)(rng->seed >> 32),
-                                                           rng->iter0, frame_utt, frame_idx, NT * n_chains, n_chains, L,
+                                                           rng->iter0, rng->iter0_frame, frame_utt, frame_idx, NT * n_chains, n_chains, L,
                                                            n_iter, eps, u);
     return check_launch("rng_dump_kernel");
 }

@@ -15,6 +15,7 @@ from __future__ import annotations
 
 import ctypes as C
 import dataclasses
+import math
 import os
 from typing import Optional, Sequence
 
@@ -172,6 +173,7 @@ class RaggedBatch:
         if len(ids) != self.B:
             raise ValueError("utt_ids length mismatch")
         self.fr_off_host = off
+        self.utt_ids_host = ids
         self.fr_off = torch.from_numpy(off).to(device)
         self.utt_ids = torch.from_numpy(ids).to(device)
         local = np.repeat(np.arange(self.B, dtype=np.int32), n)
@@ -278,6 +280,8 @@ class McemConfig:
     fuse_wstat: bool = True      # tc only: per-frame statistics of the W update instead of a pass over Vs
     emit_vs: bool = True         # tc only: the sampler writes the kept samples' variances itself (BF16); False: FP32 decode
     w_partials: bool = True      # with emit_vs: reduce the W-update sums inside the statistics kernel (no A1 / A2 round trip)
+    stop_tol: Optional[float] = None   # per-utterance stopping (check_stop, McemEngine.run); None: every utterance runs niter
+    stop_window: int = 10              # EM iterations per window of the stopping test
 
 
 class InjectedDraws:
@@ -327,6 +331,7 @@ class McemEngine:
     """EM driver for one ragged batch (replaces ``EM.run`` + ``MCEM_*`` of packages/models/mcem.py)."""
 
     def __init__(self, weights: VaeWeights, cfg: McemConfig, device):
+        check_stop(cfg)
         self.dev = _require_cuda(device)
         self.w = weights
         self.cfg = cfg
@@ -346,6 +351,9 @@ class McemEngine:
         self.kernel_launches = 0
         self.timing = False          # when True, CUDA events bracket every stage (read with stage_times_ms())
         self._events = []
+        self._iter0_frame = None     # per-frame Philox iteration base of the next sample_posterior call (final filter of run)
+        self.order = None            # after a run with stopping: slot -> caller's utterance index of the per-frame state
+        self.n_iter = None           # after a run: EM iterations of every utterance, caller's order
 
     class _Stage:
         def __init__(self, eng, name):
@@ -468,6 +476,7 @@ class McemEngine:
         rng = _lib.DvaeRng()
         rng.seed = cfg.seed & 0xFFFFFFFFFFFFFFFF
         rng.iter0 = self.mh_iter0
+        rng.iter0_frame = None if self._iter0_frame is None else self._iter0_frame.data_ptr()
         eps = u = None
         if draws is not None:
             eps, u = draws.mh_draws(self.mh_calls, keep + burn, chains, L)
@@ -610,6 +619,10 @@ class McemEngine:
         cps = check_checkpoints(checkpoints, self.cfg.niter)
         if cps and draws is not None:
             raise ValueError("checkpoints need the engine's own random numbers, not injected draws")
+        check_stop(self.cfg, draws, cps)
+        self.order, self.n_iter = None, np.full(self.batch.B, self.cfg.niter, np.int64)
+        if self.cfg.stop_tol is not None:
+            return self._run_stopping()
         for it in range(self.cfg.niter):
             self.e_step(draws)
             self.m_step(it)
@@ -619,6 +632,109 @@ class McemEngine:
         if on_checkpoint is not None and self.cfg.niter in cps:
             on_checkpoint(self.cfg.niter)
         return self.cost
+
+    def _run_stopping(self):
+        """``run`` with per-utterance stopping (``McemConfig.stop_tol``, test in ``dvae_em_stop_check``).
+
+        The batch is kept as ``[active | parked]`` in the full-size buffers.  After each EM iteration ``n >= 2 stop_window``
+        the device test flags the active utterances (one synchronisation); the active range is then stably partitioned into
+        ``[continuing | just stopped]`` (``dvae_permute_rows`` through a scratch buffer) and the E- and M-steps run on the
+        shorter prefix, whose ``RaggedBatch`` keeps the utterances' own ids, so their draws do not change.  A stopped
+        utterance records the MH iteration counter at its stop; the one final filter over the whole batch starts every frame
+        from its utterance's counter (``DvaeRng.iter0_frame``), which makes its output that of a run with ``niter = n_u``.
+        Returns the cost ``[niter][B]`` in the caller's column order, NaN after each utterance's last iteration.  The
+        per-frame state (``H``, ``g``, ``Z``, ``S_hat``, ...) stays in slot order: slot ``i`` is utterance ``order[i]`` and
+        ``batch`` is the permuted batch."""
+        cfg, full = self.cfg, self.batch
+        B, w, niter = full.B, cfg.stop_window, cfg.niter
+        self.cost.fill_(math.nan)
+        order = np.arange(B)
+        n_iter = np.full(B, niter, np.int64)
+        iter0 = np.zeros(B, np.int64)                     # MH counter at each utterance's stop, caller's order
+        flags = self._get("stop_flags", (B,), torch.uint8)
+        self._stop_moved = set()                           # caller-owned inputs already replaced by engine buffers
+        b_act = B
+        for it in range(niter):
+            self.e_step()
+            self.m_step(it)
+            n = it + 1
+            if n < 2 * w or n == niter:
+                continue
+            with self.stage("stop_check"):
+                _lib.call("dvae_em_stop_check", C.c_void_p(self.cost.data_ptr()), B, b_act, n, w, float(cfg.stop_tol), _p(flags),
+                          _stream())
+            stop = flags[:b_act].cpu().numpy().astype(bool)          # synchronises
+            if not stop.any():
+                continue
+            n_iter[order[:b_act][stop]] = n
+            iter0[order[:b_act][stop]] = self.mh_iter0
+            keep = np.flatnonzero(~stop)
+            if len(keep) == 0:
+                b_act = 0
+                break
+            perm = np.concatenate([keep, np.flatnonzero(stop)])
+            if np.any(perm != np.arange(b_act)):
+                with self.stage("stop_permute"):
+                    self._permute_active(perm, n)
+                order[:b_act] = order[:b_act][perm]
+            b_act = len(keep)
+            self.batch = RaggedBatch(full.n_frames[order[:b_act]], self.dev, full.utt_ids_host[order[:b_act]])
+        iter0[order[:b_act]] = self.mh_iter0
+        self.batch = RaggedBatch(full.n_frames[order], self.dev, full.utt_ids_host[order])
+        per_frame = np.repeat(iter0[order], full.n_frames[order]).astype(np.uint32)
+        self._iter0_frame = torch.from_numpy(per_frame).to(self.dev)
+        try:
+            self.wiener()
+        finally:
+            self._iter0_frame = None
+        out = self._get("cost_out", self.cost.shape, torch.float64)
+        inv = np.empty(B, np.int32)
+        inv[order] = np.arange(B, dtype=np.int32)
+        inv_d = torch.from_numpy(inv).to(self.dev)
+        with self.stage("stop_permute"):
+            permute_rows([(self.cost, out, inv_d, B, 8, niter, 8 * B)])
+        self.cost, self.order, self.n_iter = out, order, n_iter
+        return out
+
+    def _permute_active(self, perm, n):
+        """Move the active utterances' state so that slot ``i`` holds what slot ``perm[i]`` held: per-frame, per-chain-row and
+        per-utterance arrays and the ``n`` cost rows written so far, gathered into a scratch buffer sized for the full batch
+        (one ``dvae_permute_rows`` launch) and copied back.  The inputs ``X`` / ``P`` / ``y`` belong to the caller: on their
+        first move they are replaced by engine buffers instead of being overwritten."""
+        b, C_ = self.batch, self.cfg.n_chains
+        off = b.fr_off_host
+        fmap = np.concatenate([np.arange(off[u], off[u + 1]) for u in perm])
+        cmap = (fmap[:, None] * C_ + np.arange(C_)).reshape(-1)
+        B_full = self.cost.shape[1]
+        cost_map = np.concatenate([perm, np.arange(len(perm), B_full)])
+        maps = torch.from_numpy(np.concatenate([fmap, cmap, perm, cost_map]).astype(np.int32)).to(self.dev)
+        mf, mc, mu, mk = torch.split(maps, [len(fmap), len(cmap), len(perm), B_full])
+        rows = {"f": (mf, b.NT), "c": (mc, b.NT * C_), "u": (mu, b.B)}
+        arrays = [(k, kind) for k, kind in (("X", "f"), ("P", "f"), ("Vb", "f"), ("H", "f"), ("g", "f"), ("kscale", "f"),
+                                            ("ybias", "f"), ("y", "f"), ("Z", "c"), ("n_accept", "c"), ("W", "u"))
+                  if getattr(self, k) is not None]
+        sizes = [getattr(self, k).numel() * getattr(self, k).element_size() for k, _ in arrays] + [self.cost.numel() * 8]
+        offs = np.concatenate([[0], np.cumsum([(x + 15) // 16 * 16 for x in sizes])])
+        scratch = self._get("stop_scratch", (int(offs[-1]),), torch.uint8)
+        jobs = []
+        for (k, kind), o in zip(arrays, offs):
+            t = getattr(self, k)
+            m, nr = rows[kind]
+            jobs.append((t, scratch[o:], m, nr, t.numel() * t.element_size() // t.shape[0], 1, 0))
+        jobs.append((self.cost, scratch[offs[-2]:], mk, B_full, 8, n, 8 * B_full))
+        permute_rows(jobs)
+        for k, (t, part, _, nr, rb, rep, pitch) in zip([k for k, _ in arrays] + ["cost"], jobs):
+            nb = nr * rb if rep == 1 else rep * pitch
+            target = t
+            if k in ("X", "P", "y") and k not in self._stop_moved:
+                target = self._get("stop_" + k, t.shape, t.dtype)
+                _bytes(target)[nb:].copy_(_bytes(t)[nb:])          # the parked tail
+                if k == "y" and self.tc_y is t:
+                    self.tc_y = target
+                setattr(self, k, target)
+                self._stop_moved.add(k)
+            _bytes(target)[:nb].copy_(part[:nb])
+        self.kernel_launches += 1
 
     def _side_filter(self, n, on_checkpoint):
         """The final filter from the current state, ``on_checkpoint(n)``, then the state as it was before the filter.  The
@@ -644,6 +760,38 @@ class McemEngine:
         self.n_accept.copy_(acc0)
         for k, v in saved.items():
             setattr(self, k, v)
+
+
+def check_stop(cfg: McemConfig, draws=None, checkpoints: Sequence[int] = ()):
+    """``ValueError`` when ``cfg.stop_tol`` is set together with something per-utterance stopping cannot serve: a negative or
+    non-finite tolerance, ``stop_window < 1``, injected draws (they are indexed by call, and the final filter of a stopping
+    run serves utterances stopped at different calls) or checkpoints.  No device work."""
+    tol = cfg.stop_tol
+    if tol is None:
+        return
+    if isinstance(tol, bool) or not isinstance(tol, (int, float, np.integer, np.floating)) or not math.isfinite(tol) or tol < 0:
+        raise ValueError("stop_tol must be a finite number >= 0 or None, got %r" % (tol,))
+    win = cfg.stop_window
+    if isinstance(win, bool) or not isinstance(win, (int, np.integer)) or win < 1:
+        raise ValueError("stop_window must be an integer >= 1, got %r" % (win,))
+    if draws is not None:
+        raise ValueError("stop_tol needs the engine's own random numbers, not injected draws")
+    if tuple(checkpoints):
+        raise ValueError("stop_tol cannot be combined with score_at / checkpoints")
+
+
+def _bytes(t: torch.Tensor) -> torch.Tensor:
+    return t.view(-1).view(torch.uint8)
+
+
+def permute_rows(jobs):
+    """One ``dvae_permute_rows`` launch over ``(src, dst, map, n_rows, row_bytes, n_rep, pitch)`` jobs (device tensors; ``map``
+    int32): ``dst`` row ``i`` of every plane = ``src`` row ``map[i]``."""
+    arr = (_lib.DvaePermuteJob * max(1, len(jobs)))()
+    for j, (src, dst, m, n_rows, row_bytes, n_rep, pitch) in zip(arr, jobs):
+        j.src, j.dst, j.map = src.data_ptr(), dst.data_ptr(), m.data_ptr()
+        j.n_rows, j.row_bytes, j.n_rep, j.pitch = int(n_rows), int(row_bytes), int(n_rep), int(pitch)
+    _lib.call("dvae_permute_rows", arr, len(jobs), _stream())
 
 
 def check_checkpoints(checkpoints: Sequence[int], niter: int) -> tuple:
@@ -737,6 +885,11 @@ class Enhancer:
         X, P = stft_batch(x_dev, x_off, x_len, batch, self.n_fft, self.hop)
         eng.init_parameters(X, P, batch, y, draws)
         cost = eng.run(draws, checkpoints, on_checkpoint)
+        if eng.order is not None:            # stopping moved the frames: write every utterance through its slot's offset / length
+            o = torch.from_numpy(eng.order.astype(np.int32)).to(self.dev)
+            off_p, len_p = eng._get("x_off_perm", (batch.B,), torch.int64), eng._get("x_len_perm", (batch.B,), torch.int32)
+            permute_rows([(x_off, off_p, o, batch.B, 8, 1, 0), (x_len, len_p, o, batch.B, 4, 1, 0)])
+            batch, x_off, x_len = eng.batch, off_p, len_p
         s_dev = istft_batch(eng.S_hat, batch, x_off, x_len, total, max_len, self.n_fft, self.hop,
                             out=eng._get("s_out", (total,)))
         n_dev = istft_batch(eng.N_hat, batch, x_off, x_len, total, max_len, self.n_fft, self.hop,
@@ -787,6 +940,7 @@ class Enhancer:
         next call on this Enhancer (clone them to keep them).
         """
         eng, dev = self.engine, self.dev
+        check_stop(eng.cfg, draws, score_at)
         B = len(x_list)
         lens = np.array([len(x) for x in x_list], np.int32)
         if np.any(lens < 1):

@@ -20,14 +20,16 @@ Behaviour carried over on purpose (SURVEY §3.2):
 Extra keyword-only knobs (not in the reference): ``sampler`` ("auto": tcgen05 BF16 kernels when the decoder has the
 shipped shape, else "fp32"; "fp32": exact CUDA-core decoder; "tc": force the tensor-core kernels),
 ``n_chains``, ``seed`` and ``rng`` ("philox": counter-based draws on the device; "torch": the reference's own draw
-order taken from torch's CPU generator, for like-for-like comparisons).
+order taken from torch's CPU generator, for like-for-like comparisons), ``stop_tol`` / ``stop_window`` (stop the EM loop
+once the cost has converged, ``McemConfig.stop_tol``; ``niter`` is then the cap, ``run()`` returns the cost NaN-padded to
+``(niter,)`` and ``n_iter`` holds the iterations run; Philox draws only).
 """
 from __future__ import annotations
 
 import numpy as np
 import torch
 
-from ...engine import McemConfig, McemEngine, RaggedBatch, TorchCpuDraws, VaeWeights, _ld_for, _p, _stream
+from ...engine import McemConfig, McemEngine, RaggedBatch, TorchCpuDraws, VaeWeights, _ld_for, _p, _stream, check_stop
 from ... import _lib
 
 
@@ -42,7 +44,7 @@ class _MCEM:
     _variant = None
 
     def __init__(self, niter, nsamples_E_step=10, burnin_E_step=30, nsamples_WF=25, burnin_WF=75, var_RW=0.01, *,
-                 sampler="auto", n_chains=1, seed=0, rng="philox"):
+                 sampler="auto", n_chains=1, seed=0, rng="philox", stop_tol=None, stop_window=10):
         self.niter = niter
         self.nsamples_E_step, self.burnin_E_step = nsamples_E_step, burnin_E_step
         self.nsamples_WF, self.burnin_WF = nsamples_WF, burnin_WF
@@ -50,6 +52,10 @@ class _MCEM:
         self.sampler, self.n_chains, self.seed, self.rng = sampler, n_chains, seed, rng
         if rng not in ("philox", "torch"):
             raise ValueError("rng must be 'philox' or 'torch'")
+        self.stop_tol, self.stop_window = stop_tol, stop_window
+        if stop_tol is not None and rng == "torch":
+            raise ValueError("stop_tol needs rng='philox': the reference's draw order cannot serve utterances stopped early")
+        check_stop(McemConfig(niter=niter, stop_tol=stop_tol, stop_window=stop_window))
         self._engine = None
         self._weights_key = None
 
@@ -88,7 +94,8 @@ class _MCEM:
         if self._engine is None or self._weights_key != key or self._cfg_rank != (nmf_rank, eps):
             (kE, bE), (kW, bW) = self.schedule()
             cfg = McemConfig(niter=self.niter, keep_E=kE, burn_E=bE, keep_WF=kW, burn_WF=bW, var_rw=self.var_RW,
-                             nmf_rank=nmf_rank, eps=eps, n_chains=self.n_chains, seed=self.seed, sampler=self.sampler)
+                             nmf_rank=nmf_rank, eps=eps, n_chains=self.n_chains, seed=self.seed, sampler=self.sampler,
+                             stop_tol=self.stop_tol, stop_window=self.stop_window)
             self._weights = VaeWeights(sd, self._variant, dev, prefix=_find_prefix(sd))
             self._engine = McemEngine(self._weights, cfg, dev)
             self._weights_key, self._cfg_rank = key, (nmf_rank, eps)
@@ -122,6 +129,11 @@ class _MCEM:
             self.S_hat = np.ascontiguousarray(eng.S_hat[:, :F].t().cpu().numpy())
             self.N_hat = np.ascontiguousarray(eng.N_hat[:, :F].t().cpu().numpy())
             return cost[:, 0].cpu().numpy().astype(np.float64)
+
+    @property
+    def n_iter(self):
+        """EM iterations the last ``run()`` executed (``niter`` unless ``stop_tol`` stopped it earlier)."""
+        return int(self._engine.n_iter[0])
 
     # ---- state exposed with the reference's shapes
     @property

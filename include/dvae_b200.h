@@ -31,7 +31,7 @@
 extern "C" {
 #endif
 
-#define DVAE_ABI_VERSION 2
+#define DVAE_ABI_VERSION 3          /* 3: DvaeRng.iter0_frame appended */
 #define DVAE_ERR_ARG (-1)
 #define DVAE_MAX_LAYERS 6
 #define DVAE_MAX_L 64          /* latent dimension limit of the Metropolis-Hastings kernels */
@@ -65,6 +65,8 @@ typedef struct DvaeRng {
     uint32_t reserved;
     const float* eps;          /* nullable */
     const float* u;            /* nullable; required when eps is given */
+    const uint32_t* iter0_frame;   /* nullable [NT] (device): per-frame replacement of iter0, so frames whose EM loops stopped
+                                      at different iterations draw their own counters in one call; Philox mode only */
 } DvaeRng;
 
 int dvae_version(void);
@@ -318,6 +320,29 @@ int dvae_vad_labels(const float* x, const int64_t* x_off, const int32_t* x_len, 
                     void* stream);
 int dvae_ibm_labels(const void* S, const int32_t* frame_utt, const int64_t* fr_off, int B, int64_t NT, int F, int ld,
                     float eps, float ibm_threshold_db, const float* vad, float* mask, void* ws, void* stream);
+
+/* ---- per-utterance stopping of the EM loop ----
+ * dvae_em_stop_check: after EM iteration n (1-based) with window w (n >= 2w), for the columns u < B_active of the cost matrix
+ * cost[niter][ld_cost] (row k = the costs after iteration k, 0-based): m_old = (cost[n-2w][u] + ... + cost[n-w-1][u]) / w and
+ * m_new = (cost[n-w][u] + ... + cost[n-1][u]) / w, both summed in ascending k in double; stop[u] = 1 when
+ * m_old - m_new <= tol * |m_new| (never when a cost is NaN), else 0. */
+int dvae_em_stop_check(const double* cost, int ld_cost, int B_active, int n, int w, double tol, uint8_t* stop, void* stream);
+
+/* dvae_permute_rows: gathers of rows by index maps, every job of the list in one launch:
+ *   dst + r * pitch + i * row_bytes <- src + r * pitch + map[i] * row_bytes   for i < n_rows, r < n_rep.
+ * row_bytes a positive multiple of 4; 16-byte vector copies when row_bytes, pitch, src and dst are multiples of 16.  src and dst
+ * must not overlap.  jobs [host]: up to DVAE_PERMUTE_MAX_JOBS. */
+#define DVAE_PERMUTE_MAX_JOBS 16
+typedef struct DvaePermuteJob {
+    const void* src;
+    void* dst;
+    const int32_t* map;        /* [n_rows] source row of each destination row */
+    int64_t n_rows;
+    int64_t row_bytes;
+    int64_t n_rep;             /* >= 1 planes `pitch` bytes apart (the columns of a row-major matrix: row_bytes = element size) */
+    int64_t pitch;
+} DvaePermuteJob;
+int dvae_permute_rows(const DvaePermuteJob* jobs, int n_jobs, void* stream);
 
 /* uniform [eps,1) initialisation of W, H and g = 1 from Philox (mcem.py:42-44: max(rand, eps)) */
 int dvae_nmf_init(uint64_t seed, const int32_t* utt_ids /*[B] global ids*/, const int64_t* fr_off, int B, int64_t NT, int F,
