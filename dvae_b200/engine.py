@@ -277,9 +277,7 @@ class McemConfig:
     n_chains: int = 1
     seed: int = 0
     sampler: str = "fp32"        # "fp32": CUDA-core exact mode; "tc": tcgen05 BF16 kernels; "auto": tc when supported
-    fuse_wstat: bool = True      # tc only: per-frame statistics of the W update instead of a pass over Vs
-    emit_vs: bool = True         # tc only: the sampler writes the kept samples' variances itself (BF16); False: FP32 decode
-    w_partials: bool = True      # with emit_vs: reduce the W-update sums inside the statistics kernel (no A1 / A2 round trip)
+    w_partials: bool = True      # emission route: reduce the W-update sums inside the statistics kernel (no A1 / A2 round trip)
     stop_tol: Optional[float] = None   # per-utterance stopping (check_stop, McemEngine.run); None: every utterance runs niter
     stop_window: int = 10              # EM iterations per window of the stopping test
 
@@ -327,8 +325,24 @@ def tc_supported(w: "VaeWeights") -> bool:
     return dims[-1] == 513 and len(dims) in (3, 4) and all(d == 128 for d in dims[1:-1]) and w.z_dim in (16, 32)
 
 
+def mcem_route(cfg: McemConfig, F: int) -> tuple:
+    """``(e_route, filter_chunk)`` for a resolved ``cfg.sampler`` and ``F`` decoder outputs; no device work.  E-step routes: "emit"
+    (the tcgen05 sampler writes the variances, BF16; a frame's chains share a 128-row tile of the M-step kernels), "stats" (FP32
+    ``Vs`` + W-update statistics in one decode pass), "decode" (FP32 ``Vs``).  ``filter_chunk``: samples per fused decode of the
+    final filter; 0: FP32 decode in frame chunks."""
+    tc, c = cfg.sampler == "tc", cfg.n_chains
+    if tc and cfg.nmf_rank <= 10 and cfg.keep_E in (10, 30) and F == 513 and (c == 1 or (c <= 128 and c & (c - 1) == 0 and cfg.w_partials)):
+        route = "emit"
+    elif tc and cfg.nmf_rank <= 10 and c * cfg.keep_E % 10 == 0:
+        route = "stats"
+    else:
+        route = "decode"
+    return route, next((k for k in (30, 25, 10) if c * cfg.keep_WF % k == 0), 0) if tc else 0
+
+
 class McemEngine:
-    """EM driver for one ragged batch (replaces ``EM.run`` + ``MCEM_*`` of packages/models/mcem.py)."""
+    """EM driver for one ragged batch (replaces ``EM.run`` + ``MCEM_*`` of packages/models/mcem.py).  ``route`` /
+    ``filter_chunk`` (``mcem_route``) are plain attributes, not settings: tests override ``route`` to compare two routes."""
 
     def __init__(self, weights: VaeWeights, cfg: McemConfig, device):
         check_stop(cfg)
@@ -346,8 +360,10 @@ class McemEngine:
             raise ValueError("latent dimension above %d" % _lib.MAX_L)
         self.F = weights.x_dim
         self.ld = _ld_for(self.F)
+        self.route, self.filter_chunk = mcem_route(cfg, self.F)
         self._buf = {}
         self.mh_calls = 0
+        self.mh_rows = 0             # decoder rows the sampler evaluated (one per chain and MH iteration), all calls
         self.kernel_launches = 0
         self.timing = False          # when True, CUDA events bracket every stage (read with stage_times_ms())
         self._events = []
@@ -438,9 +454,9 @@ class McemEngine:
         self.n_accept.zero_()
         self.mh_calls = 0
         self.mh_iter0 = 0
-        self.vst_R = 0                    # > 0: the last E-step's variances live in the sampler's emission (VsT / vs_idx)
+        self.VsT = self.vs_idx = self.wstat = self.wpart = None    # the last E-step's emission and W-update statistics
         self._Vs = None
-        self._last_Zs = None
+        self._last_Zs = None              # the final filter's samples, from the filter until the next E-step
         self.cost = self._get("cost", (cfg.niter, B), torch.float64)
         self.kernel_launches = 0
 
@@ -452,18 +468,17 @@ class McemEngine:
         return self._get("Vs", (max(b.NT * cfg.n_chains * cfg.keep_E, cfg.n_chains * cfg.keep_WF), self.ld))
 
     @property
+    @_on_device
     def Vs(self):
-        """Speech variances of the last E-step's kept samples, ``[NT][R][ld]`` FP32 (the reference's ``self.Vs`` (R,F,N) up
-        to layout).  When they only exist in the sampler's BF16 emission they are unpacked on demand."""
-        if self._Vs is None and self.vst_R:
-            with torch.cuda.device(self.dev):
-                from . import tc
-                self._Vs = tc.vst_unpack(self, self.vst_R)
-        elif self._Vs is None and getattr(self, "_last_Zs", None) is not None:
-            Zs = self._last_Zs                     # the final filter never materialises its samples: decode them on demand
-            out = torch.zeros((self.batch.NT, Zs.shape[1], self.ld), dtype=torch.float32, device=self.dev)
-            self.decode_samples(Zs, 0, self.batch.NT, out)
+        """Speech variances of the last sampled set (the filter's until the next E-step), ``[NT][R][ld]`` FP32: the reference's
+        ``self.Vs`` (R,F,N) up to layout.  The filter's samples and the "emit" route's BF16 emission are decoded on demand."""
+        if self._Vs is None and self._last_Zs is not None:
+            out = torch.zeros((self.batch.NT, self._last_Zs.shape[1], self.ld), dtype=torch.float32, device=self.dev)
+            self.decode_samples(self._last_Zs, 0, self.batch.NT, out)
             self._Vs = out
+        elif self._Vs is None and self.VsT is not None:      # only an E-step on the "emit" route leaves an emission behind
+            from . import tc
+            self._Vs = tc.vst_unpack(self, self.cfg.keep_E)
         return self._Vs
 
     # -- one sample_posterior call (mcem.py:207-277): returns kept samples [NT][C*keep][L]
@@ -496,7 +511,7 @@ class McemEngine:
                           _p(b.frame_gid), _p(b.frame_idx), _p(self.Z), _p(Zs), b.NT, self.F, self.ld, L, C_, burn, keep,
                           float(cfg.var_rw), C.byref(rng), _p(self.n_accept), _p(a_trace), _p(ws), _stream())
                 self.kernel_launches += (keep + burn + 1) * (len(w.dec.dims) - 1 + 1)
-        self.mh_rows = getattr(self, "mh_rows", 0) + chains * (keep + burn + 1)
+        self.mh_rows += chains * (keep + burn + 1)
         self.mh_calls += 1
         self.mh_iter0 += keep + burn
         return Zs
@@ -520,31 +535,25 @@ class McemEngine:
 
     @_on_device
     def e_step(self, draws=None):
-        """E-step (mcem.py:292-308): sample, keep the last state, decode the kept samples.  On the tensor-core path (one chain
-        per frame, or a power-of-two number of them) the sampler emits the variances itself (BF16) and only the statistics
-        of the W update are computed here; otherwise the kept samples are decoded into FP32 ``Vs``."""
+        """E-step (mcem.py:292-308): sample, keep the last state, and hand the kept samples to the M-step along ``route``
+        (``mcem_route``): the sampler's own BF16 emission + the W-update statistics, or FP32 ``Vs`` with or without them."""
         cfg = self.cfg
-        self.wstat, self.wpart, self._Vs, self.vst_R = None, None, None, 0
-        if cfg.sampler == "tc":
-            from . import tc
-            if tc.vst_supported(self, cfg.keep_E):
-                self.sample_posterior(cfg.keep_E, cfg.burn_E, draws, emit=True)
-                self.vst_R, self.R = cfg.keep_E, cfg.n_chains * cfg.keep_E      # kept per chain, samples per frame
-                with self.stage("decode"):
-                    if cfg.w_partials:
-                        self.wpart = tc.vst_w_partials(self, self.vst_R)
-                    else:
-                        self.wstat = tc.vst_frame_stats(self, self.vst_R)
-                return
-        Zs = self.sample_posterior(cfg.keep_E, cfg.burn_E, draws)
-        self.R = Zs.shape[1]
-        self._Vs = self.Vs_flat[: self.batch.NT * self.R].view(self.batch.NT, self.R, self.ld)
-        if cfg.sampler == "tc" and self.R % 10 == 0 and cfg.nmf_rank <= 10 and cfg.fuse_wstat:
-            from . import tc
-            with self.stage("decode"):
-                self.wstat = tc.decode_stats_tc(self, Zs, self._Vs)
-        else:
+        self.wstat, self.wpart, self._Vs, self._last_Zs = None, None, None, None
+        self.R = cfg.n_chains * cfg.keep_E                                  # samples per frame
+        Zs = self.sample_posterior(cfg.keep_E, cfg.burn_E, draws, emit=self.route == "emit")
+        if self.route != "emit":
+            self._Vs = self.Vs_flat[: self.batch.NT * self.R].view(self.batch.NT, self.R, self.ld)
+        if self.route == "decode":
             self.decode_samples(Zs, 0, self.batch.NT, self._Vs)
+            return
+        from . import tc
+        with self.stage("decode"):
+            if self.route == "stats":
+                self.wstat = tc.decode_stats_tc(self, Zs, self._Vs)
+            elif cfg.w_partials:
+                self.wpart = tc.vst_w_partials(self, cfg.keep_E)
+            else:
+                self.wstat = tc.vst_frame_stats(self, cfg.keep_E)
 
     @_on_device
     def m_step(self, it: int):
@@ -553,18 +562,18 @@ class McemEngine:
         ws = self._get("nmf_ws", (int(need),))
         st = self._buf.get("tc_status")
         with self.stage("mstep"):
-            if self.vst_R:
+            if self.route == "emit":
                 from . import tc
                 w = self.w
                 _lib.call("dvae_nmf_mstep_vst", w.dec_tc.ref, _p(tc.decoder_image(w)), w.z_dim, w.tc_y_dim, _p(self.P), _p(self.VsT),
-                          _p(self.vs_idx), self.vst_R, _p(self.W), _p(self.H), _p(self.g), _p(self.Vb),
+                          _p(self.vs_idx), cfg.keep_E, _p(self.W), _p(self.H), _p(self.g), _p(self.Vb),
                           C.c_void_p(self.cost[it].data_ptr()), _p(b.fr_off), b.B, b.NT, cfg.nmf_rank, self.ld, b.max_frames,
                           _p(ws), _p(self.wstat), _p(self.wpart),
                           _p(b.segments(n_chains=cfg.n_chains)[2]) if self.wpart is not None else None, cfg.n_chains, _p(st), _stream())
             else:
                 _lib.call("dvae_nmf_mstep", _p(self.P), _p(self._Vs), self.R, _p(self.W), _p(self.H), _p(self.g), _p(self.Vb),
                           C.c_void_p(self.cost[it].data_ptr()), _p(b.fr_off), _p(b.frame_utt), b.B, b.NT, self.F, cfg.nmf_rank,
-                          self.ld, b.max_frames, _p(ws), _p(getattr(self, "wstat", None)), _p(st), _stream())
+                          self.ld, b.max_frames, _p(ws), _p(self.wstat), _p(st), _stream())
         self.kernel_launches += 4
 
     @_on_device
@@ -572,12 +581,11 @@ class McemEngine:
         """``compute_WF(sample=True)`` + the mask application of ``EM.run`` (mcem.py:310-329, 176-177)."""
         cfg, b = self.cfg, self.batch
         Zs = self.sample_posterior(cfg.keep_WF, cfg.burn_WF, draws)
-        self._Vs, self.vst_R, self._last_Zs = None, 0, Zs
-        R = Zs.shape[1]
+        self._Vs, self._last_Zs = None, Zs
+        R, chunk = Zs.shape[1], self.filter_chunk
         WFs = self._get("WFs", (b.NT, self.ld))
         WFn = self._get("WFn", (b.NT, self.ld))
-        chunk = next((c for c in (30, 25, 10) if R % c == 0), 0)
-        if cfg.sampler == "tc" and chunk:
+        if chunk:
             # fused: the filter samples are decoded chunk by chunk straight into A1 = sum_r 1 / Vx; the masks follow from
             # mean_r g Vs / Vx = 1 - Vb A1 / R, so none of the R x F x N variances is written to memory
             from . import tc
@@ -746,8 +754,7 @@ class McemEngine:
         acc0 = self._get("n_accept_trace", self.n_accept.shape, torch.int32)
         Z0.copy_(self.Z)
         acc0.copy_(self.n_accept)
-        names = ("mh_calls", "mh_iter0", "mh_rows", "_Vs", "vst_R", "_last_Zs", "VsT", "vs_idx")
-        saved = {k: getattr(self, k) for k in names if hasattr(self, k)}
+        saved = {k: getattr(self, k) for k in ("mh_calls", "mh_iter0", "mh_rows", "_Vs", "_last_Zs", "VsT", "vs_idx")}
         with self.stage("trace"):
             timing, self.timing = self.timing, False
             try:

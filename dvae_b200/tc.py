@@ -83,15 +83,6 @@ def row_scale(eng):
     return k
 
 
-def vst_supported(eng, keep):
-    """The sampler's own emission of the kept samples' variances serves up to 31 kept samples per chain and (for the fused
-    M-step kernels) keep in {10, 30}, K <= 10, F = 513; several chains per frame need a power-of-two count (the chains of a
-    frame share a 128-row tile) and the segment partial sums."""
-    c = eng.cfg.n_chains
-    return ((c == 1 or (c <= 128 and c & (c - 1) == 0 and eng.cfg.w_partials)) and keep in (10, 30) and eng.cfg.nmf_rank <= 10
-            and eng.F == 513 and eng.ld == 520 and eng.cfg.fuse_wstat and eng.cfg.emit_vs)
-
-
 def mh_chain_tc(eng, Zs, keep, burn, rng, a_trace, emit=False):
     """One ``sample_posterior`` call on the tcgen05 sampler.  ``emit``: also write the kept samples' variances
     (``eng.VsT`` / ``eng.vs_idx``, see dvae_mh_chain_tc2)."""

@@ -214,10 +214,11 @@ def test_full_size_properties_configs1():
     np.testing.assert_allclose(c3, c1[lo:hi], rtol=1e-12)
 
 
-def test_multi_chain_windowed_path_matches_generic_path():
-    """4 chains x 10 kept samples = 40 samples per frame: the windowed fused decode + windowed M-step kernel against the
-    generic kernels (materialised decode, generic NMF passes) on the same draws, and the sampler's own emission with the
-    windowed emission M-step kernel (BF16 variances: looser tolerance)."""
+def test_multi_chain_routes_agree_end_to_end():
+    """4 chains x 10 kept samples = 40 samples per frame on the tensor-core sampler, one enhancement per E-step route
+    (``McemEngine.route``): "stats" (windowed fused decode + windowed M-step kernel) against "decode" (materialised decode,
+    generic NMF passes) on the same draws, and "emit" (the sampler's own emission with the windowed emission M-step kernel;
+    BF16 variances: looser tolerance)."""
     from dvae_b200.engine import Enhancer, McemConfig
     x = synth.synth_utterance(41, 1.2)[0]
     s_clean = synth.synth_utterance(41, 1.2)[1]
@@ -225,9 +226,11 @@ def test_multi_chain_windowed_path_matches_generic_path():
     sd = synth.xavier_state_dict("M2v3", 513, 16, [128, 128], 1, seed=6, out_bias=float(np.log(P0.mean())))
     y = synth.energy_vad(s_clean)
     out = {}
-    for mode, fuse, emit in (("win", True, False), ("generic", False, False), ("emit", True, True)):
-        cfg = McemConfig(niter=3, keep_E=10, burn_E=5, keep_WF=25, burn_WF=5, seed=1, n_chains=4, fuse_wstat=fuse, emit_vs=emit)
+    for mode, route in (("win", "stats"), ("generic", "decode"), ("emit", "emit")):
+        cfg = McemConfig(niter=3, keep_E=10, burn_E=5, keep_WF=25, burn_WF=5, seed=1, n_chains=4, sampler="tc")
         enh = Enhancer(sd, "M2v3", cfg, device=0)
+        assert enh.engine.route == "emit"
+        enh.engine.route = route
         s, n, c = enh.enhance([x], y_list=[y], utt_ids=[3])
         assert enh.engine.R == 40 and enh.engine.R_wf == 100
         out[mode] = (s[0].copy(), c.copy())

@@ -207,13 +207,13 @@ def test_tc_rejects_unsupported_shapes():
 
 
 @pytest.mark.parametrize("variant,keep", [("M1", 30), ("M2", 10), ("M2v3", 10)])
-def test_fused_decode_stats_and_emission_match_unfused(variant, keep):
-    """Three ways through the E-step tail on the same Philox draws: (a) decode_tc + the W kernel that reads Vs, (b)
-    dvae_decode_stats_tc (FP32 Vs + frame statistics in one pass), (c) the sampler's own BF16 emission + dvae_vst_frame_stats
-    + dvae_nmf_mstep_vst.  (b) must equal (a) to FP32 rounding; (c) carries the BF16 rounding of the stored variances
-    (2^-9 relative per value + the sampler's polynomial exp2: stated tolerance 1.2 % per variance of the first E-step, where
-    all three hold the same samples, and 2 % relative L2 on the M-step outputs of this two-iteration run, whose second
-    E-step may already take a different accept decision here and there)."""
+def test_stats_and_emit_routes_match_decode_route(variant, keep):
+    """The three E-step routes (``McemEngine.route``) on the same Philox draws: (a) "decode": decode_tc + the W kernel that
+    reads Vs, (b) "stats": dvae_decode_stats_tc (FP32 Vs + frame statistics in one pass), (c) "emit": the sampler's own BF16
+    emission + dvae_vst_w_partials or dvae_vst_frame_stats + dvae_nmf_mstep_vst.  (b) must equal (a) to FP32 rounding; (c)
+    carries the BF16 rounding of the stored variances (2^-9 relative per value + the sampler's polynomial exp2: stated
+    tolerance 1.2 % per variance of the first E-step, where all three hold the same samples, and 2 % relative L2 on the M-step
+    outputs of this two-iteration run, whose second E-step may already take a different accept decision here and there)."""
     y_dim = 0 if variant == "M1" else 1
     lens = [185, 37, 1, 64]                                     # ragged: partial tiles, one-frame utterance
     NT = sum(lens)
@@ -224,20 +224,21 @@ def test_fused_decode_stats_and_emission_match_unfused(variant, keep):
     sd = synth.xavier_state_dict(variant, 513, 16, [128, 128], y_dim, seed=9, out_bias=float(np.log(0.05)))
     w = VaeWeights(sd, variant, torch.device(DEV))
     out = {}
-    for mode, fuse, emit in (("unfused", False, False), ("stats", True, False), ("emit", True, True), ("emit_a1a2", True, True)):
-        cfg = McemConfig(niter=2, keep_E=keep, burn_E=5, keep_WF=3, burn_WF=3, sampler="tc", seed=3, fuse_wstat=fuse, emit_vs=emit,
-                         w_partials=(mode == "emit"))
+    for mode, route in (("decode", "decode"), ("stats", "stats"), ("emit", "emit"), ("emit_a1a2", "emit")):
+        cfg = McemConfig(niter=2, keep_E=keep, burn_E=5, keep_WF=3, burn_WF=3, sampler="tc", seed=3, w_partials=(mode == "emit"))
         eng = McemEngine(w, cfg, DEV)
+        assert eng.route == "emit"                              # what these shapes run; the other routes are forced
+        eng.route = route
         eng.init_parameters(X, P, RaggedBatch(lens, DEV), y)
         for it in range(2):
             eng.e_step()
-            assert ((eng.wstat is not None) or (eng.wpart is not None)) == fuse and (eng.vst_R > 0) == emit and (eng.wpart is not None) == (mode == "emit")
+            assert ((eng.wstat is not None) or (eng.wpart is not None)) == (route != "decode") and (eng.VsT is not None) == (route == "emit") and (eng.wpart is not None) == (mode == "emit")
             if it == 0:
                 vs = eng.Vs.clone()
             eng.m_step(it)
         tc.check_status(eng)
         out[mode] = (vs.cpu(), eng.W.cpu().clone(), eng.H.cpu().clone(), eng.g.cpu().clone(), eng.cost.cpu().clone())
-    a = out["unfused"]
+    a = out["decode"]
     for i in (1, 2, 3, 4):                            # the two W reductions of the emission path differ by summation order only
         assert ((out["emit"][i] - out["emit_a1a2"][i]).double().norm() / out["emit_a1a2"][i].double().norm()).item() <= 1e-5
     for mode, tol_vs, tol in (("stats", 1e-5, 1e-4), ("emit", 1.2e-2, 2e-2)):
@@ -254,11 +255,12 @@ def test_fused_decode_stats_and_emission_match_unfused(variant, keep):
 
 
 @pytest.mark.parametrize("variant,keep,chains", [("M2v3", 10, 16), ("M2", 10, 2), ("M1", 30, 4)])
-def test_multi_chain_emission_matches_decoded_samples(variant, keep, chains):
-    """Several chains per frame: the sampler's emission + dvae_vst_w_partials + the windowed emission M-step kernel against the
-    windowed FP32 decode (dvae_decode_stats_win_tc) + its M-step kernel on the same Philox draws.  The first E-step holds the
-    same samples on both paths (BF16 storage: 1.2 % per variance); M-step outputs after it within 0.5 % relative L2, after a
-    second iteration (accept decisions may differ here and there) within 2 %."""
+def test_multi_chain_emit_route_matches_stats_route(variant, keep, chains):
+    """Several chains per frame, "emit" route against "stats" route: the sampler's emission + dvae_vst_w_partials + the
+    windowed emission M-step kernel against the windowed FP32 decode (dvae_decode_stats_win_tc) + its M-step kernel on the
+    same Philox draws.  The first E-step holds the same samples on both paths (BF16 storage: 1.2 % per variance); M-step
+    outputs after it within 0.5 % relative L2, after a second iteration (accept decisions may differ here and there) within
+    2 %."""
     y_dim = 0 if variant == "M1" else 1
     lens = [70, 37, 1, 20]
     NT = sum(lens)
@@ -269,22 +271,25 @@ def test_multi_chain_emission_matches_decoded_samples(variant, keep, chains):
     sd = synth.xavier_state_dict(variant, 513, 16, [128, 128], y_dim, seed=9, out_bias=float(np.log(0.05)))
     w = VaeWeights(sd, variant, torch.device(DEV))
     out = {}
-    for mode, emit in (("decode", False), ("emit", True)):
-        cfg = McemConfig(niter=2, keep_E=keep, burn_E=5, keep_WF=3, burn_WF=3, sampler="tc", seed=3, n_chains=chains, emit_vs=emit)
+    for route in ("stats", "emit"):
+        cfg = McemConfig(niter=2, keep_E=keep, burn_E=5, keep_WF=3, burn_WF=3, sampler="tc", seed=3, n_chains=chains)
         eng = McemEngine(w, cfg, DEV)
+        assert eng.route == "emit"
+        eng.route = route
         eng.init_parameters(X, P, RaggedBatch(lens, DEV), y)
         snap = []
         for it in range(2):
             eng.e_step()
-            assert (eng.vst_R == keep) == emit and (eng.wpart is not None) == emit and eng.R == chains * keep
+            emit = route == "emit"
+            assert (eng.VsT is not None) == emit and (eng.wpart is not None) == emit and (eng.wstat is not None) != emit and eng.R == chains * keep
             if it == 0:
                 vs = eng.Vs.clone()
                 assert tuple(vs.shape) == (NT, chains * keep, 520)
             eng.m_step(it)
             snap.append([t.cpu().clone() for t in (eng.W[..., :513], eng.H, eng.g, eng.Vb[:, :513], eng.cost[it])])
         tc.check_status(eng)
-        out[mode] = (vs.cpu(), snap)
-    a, b = out["decode"], out["emit"]
+        out[route] = (vs.cpu(), snap)
+    a, b = out["stats"], out["emit"]
     assert ((a[0][:, :, :513] - b[0][:, :, :513]).abs() / a[0][:, :, :513]).max().item() <= 1.2e-2
     for it, tol in ((0, 5e-3), (1, 2e-2)):
         for name, ref, got in zip(("W", "H", "g", "Vb", "cost"), a[1][it], b[1][it]):

@@ -206,6 +206,27 @@ def test_segment_tables_refine_tiles_and_utterances():
             assert utt_seg[0] == 0 and utt_seg[-1] == S and tile_seg[-1] == S
 
 
+@pytest.mark.parametrize("kw,F,route,chunk", [
+    (dict(keep_E=30, keep_WF=75), 513, "emit", 25),                           # bench headline, M1
+    (dict(keep_E=10, keep_WF=25), 513, "emit", 25),                           # M2 variants
+    (dict(keep_E=10, keep_WF=25, n_chains=16), 513, "emit", 25),
+    (dict(keep_E=10, keep_WF=25, w_partials=False), 513, "emit", 25),
+    (dict(keep_E=10, keep_WF=25, n_chains=2, w_partials=False), 513, "stats", 25),
+    (dict(keep_E=10, keep_WF=25, n_chains=3), 513, "stats", 25),
+    (dict(keep_E=20, keep_WF=30), 513, "stats", 30),
+    (dict(keep_E=5, keep_WF=5), 513, "decode", 0),
+    (dict(keep_E=10, keep_WF=20, nmf_rank=12), 513, "decode", 10),
+    (dict(keep_E=10, keep_WF=25, n_chains=256), 513, "stats", 25),
+    (dict(keep_E=30, keep_WF=75, sampler="fp32"), 513, "decode", 0),
+    (dict(keep_E=10, keep_WF=25, sampler="fp32"), 257, "decode", 0),
+])
+def test_mcem_route_table(kw, F, route, chunk):
+    """mcem_route: which E-step route (sampler emission / FP32 decode + statistics / FP32 decode) and which final-filter chunk
+    a configuration runs, without a device."""
+    from dvae_b200.engine import McemConfig, mcem_route
+    assert mcem_route(McemConfig(**dict(dict(sampler="tc"), **kw)), F) == (route, chunk)
+
+
 def test_emission_consumers_validate_their_arguments_before_any_launch():
     """dvae_vst_w_partials / dvae_nmf_mstep_vst: chain counts that are not a power of two <= 128, several chains without the
     segment partial sums, both or neither of fstat / wpart, a wrong sample count - all refused with a negative status and a

@@ -112,7 +112,7 @@ for tag in "BCDEFG":
         out["v%s %s" % (tag, mode)] = timed(var)
 eng.timing = False
 eng.sample_posterior(keep, burn, None, emit=True)
-eng.R = eng.vst_R = keep
+eng.R = keep
 out["frame_stats"] = timed(lambda: tc.vst_frame_stats(eng, keep))
 out["w_partials"] = timed(lambda: tc.vst_w_partials(eng, keep))
 eng.wstat, eng.wpart = None, tc.vst_w_partials(eng, keep)
