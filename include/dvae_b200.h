@@ -118,7 +118,13 @@ int dvae_nmf_vb(const float* W, const float* H, const int32_t* frame_utt, int64_
  *   cost[u] = mean_{r,f,n in u}(log Vx + P/Vx) with the new g.
  * In/out: W[B][K][ld], H[NT][K], g[NT], Vb[NT][ld] (in: product used by the E-step; out: W_new H_new before
  * normalisation, as the reference keeps it).  cost: [B] doubles, overwritten.
- * ws: dvae_nmf_workspace_floats(B, K, ld, max_frames) floats, 8-byte aligned. */
+ * ws: dvae_nmf_workspace_floats(B, K, ld, max_frames) floats, 8-byte aligned.
+ * Supported input range (this entry point, dvae_nmf_mstep_vst and the dvae_vst_* statistics passes; DESIGN section 6): every
+ * Vx = g Vs + Vb the M-step forms (E-step g and Vb, then W_new H_old, W_new H_new, g_new) lies in [2^-60, 2^60], and the
+ * samples of a bin lie within 2^+-31 of the bin's first sample.  Inside, every output is within the error model of
+ * tests/test_gpu_mstep_f64.py of float64.  Below 2^-63 the pair products x0 x1 of the shared reciprocals leave FP32's normal
+ * range, above 2^63 their reciprocal does; a wider spread overflows the cost passes' products of four samples: such inputs end
+ * in DVAE_STATUS_NONFINITE or, on the generic (IEEE reciprocal) kernels, in results that still meet the bound. */
 int64_t dvae_nmf_workspace_floats(int B, int K, int ld, int max_frames);
 int dvae_nmf_mstep(const float* P, const float* Vs, int R, float* W, float* H, float* g, float* Vb, double* cost,
                    const int64_t* fr_off, const int32_t* frame_utt, int B, int64_t NT, int F, int K, int ld,

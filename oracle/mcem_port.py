@@ -294,6 +294,96 @@ def m_step_reference(P, Vs, W, H, g):
     return dict(W=o.W, H=o.H, g=o.g, Vb=o.Vb, Vx=o.Vx, cost=o.cost_value())
 
 
+# Error model of the CUDA M-step (nmf.cu, vst.cu, decode_stats_tc.cu) against float64.  Every sum of the M-step except the
+# cost adds positive terms, so a relative error bound of the terms carries over to the sum plus u per addition along the
+# longest chain of additions; products add their factors' bounds, sqrt halves its argument's.  u = 2^-24 (FP32 rounding).
+U32 = 2.0 ** -24
+RCP_REL = 4 * U32            # 1 / Vx through the pair trick: x0 x1 (u), rcp.approx (1 ulp <= 2u), x1 * rcp (u)
+VX_IN_REL = 3 * U32          # g Vs: g E (u, emission), (g E) v (u), Vs = E v of the unpacked reference (u)
+DEPTH_F = 17                 # additions of a sum over the bins: <= 3 bins per thread (2), 5 shuffle levels, 8 warps, bin 512's term
+LG2_ABS = 2.0 ** -22         # lg2.approx.f32 absolute error (PTX ISA); one per product of up to four samples, counted per sample
+QUAD_REL = 12 * U32          # P / Vx of the cost pass: three products of four y (3u), two sums (2u), rcp.approx (2u), scaling (5u)
+# Vx = g Vs + Vb range the M-step's FP32 arithmetic handles: pair products x0 x1 stay normal (2^-126 .. 2^126 leaves the
+# reciprocal normal under .ftz), with a margin of 2^4 for R <= 256 reciprocal squares summed and multiplied by P.
+VX_MIN, VX_MAX = 2.0 ** -60, 2.0 ** 60
+BIN_SPREAD_LOG2 = 31         # the cost passes' per-bin scale: samples of a bin within 2^+-31 of the bin's first sample
+
+
+def m_step_f64(P, Vs, W, H, g, segments=None, chains=1, stats_rel=None):
+    """One M-step (mcem.py:91-153, the order of ``MCEMOracle.M_step``) in float64, with its intermediates and error bounds.
+
+    ``P`` (F,N), ``Vs`` (R,F,N), ``W`` (F,K), ``H`` (K,N), ``g`` (N,): one utterance, numpy or torch.  ``segments``: frame
+    ranges ``[(a, b), ...]`` whose W-update sums are returned separately (the layout of ``Wpart``, [S][K][2][F]).  ``chains``:
+    sample rows per frame in the W reduction (its additions run over ``N * chains`` rows).  ``stats_rel``: relative error of
+    A1 / A2 when the caller hands them to the kernels itself (FP32 rounding of these float64 values: ``U32``).
+
+    Returns float64 numpy arrays: ``W H g Vb cost`` as ``m_step_reference``, ``cost_terms`` = ln Vx + P / Vx (R,F,N), ``A1``
+    ``A2`` (F,N) with the E-step's g and Vb, ``Wnum Wden`` (F,K) = sum_n P A2 H, sum_n A1 H (``Wpart`` with segments), the
+    error-model bounds ``bound_W bound_H bound_g bound_Vb bound_A1 bound_A2 bound_Wsum`` (absolute, per element) and
+    ``bound_cost``, and for range checks ``vx_min vx_max`` over every Vx the M-step forms and ``spread_log2``, the largest
+    |log2(Vx_r / Vx_0)| of a bin in the cost pass.
+    """
+    f64 = lambda a: (a.detach().cpu().numpy() if torch.is_tensor(a) else np.asarray(a)).astype(np.float64)
+    P, Vs, W, H, g = f64(P), f64(Vs), f64(W), f64(H), f64(g)
+    R, F, N = Vs.shape
+    K = W.shape[1]
+    u = U32
+    out = {}
+    Vx0 = g * Vs + W @ H
+    A1, A2 = (1.0 / Vx0).sum(0), (1.0 / Vx0 ** 2).sum(0)
+    numW, denW = (P * A2) @ H.T, A1 @ H.T
+    Wt = W * np.sqrt(numW / denW)
+    Vx1 = g * Vs + Wt @ H
+    numH, denH = Wt.T @ (P * (Vx1 ** -2).sum(0)), Wt.T @ (Vx1 ** -1).sum(0)
+    Ht = H * np.sqrt(numH / denH)
+    Vb = Wt @ Ht
+    Vx2 = g * Vs + Vb
+    norm = np.abs(Wt).sum(0)
+    ng, dg = (P * (Vs * Vx2 ** -2).sum(0)).sum(0), (Vs * Vx2 ** -1).sum(0).sum(0)
+    gn = g * np.sqrt(ng / dg)
+    Vx3 = gn * Vs + Vb
+    terms = np.log(Vx3) + P / Vx3
+    out.update(W=Wt / norm, H=Ht * norm[:, None], g=gn, Vb=Vb, cost=terms.mean() if terms.size else 0.0, cost_terms=terms,
+               A1=A1, A2=A2, Wnum=numW, Wden=denW)
+    if segments is not None:
+        out["Wpart"] = np.stack([np.stack([(P * A2)[:, a:b] @ H[:, a:b].T, A1[:, a:b] @ H[:, a:b].T], 0).transpose(2, 0, 1)
+                                 for a, b in segments]) if len(segments) else np.zeros((0, K, 2, F))
+    # ---- relative bounds, pass by pass (all terms positive: one number per output)
+    e_vx0 = VX_IN_REL + K * u + u                                        # Vb = W H by K FMAs, then + g Vs
+    e_a1 = e_vx0 + RCP_REL + (R - 1) * u
+    e_a2 = 2 * (e_vx0 + RCP_REL) + u + (R - 1) * u
+    ea1w, ea2w = (stats_rel, stats_rel) if stats_rel is not None else (e_a1, e_a2)
+    rows = N * chains + (len(segments) if segments else 0)               # W sums: every row, then the segments in order
+    e_wsum_num, e_wsum_den = ea2w + 2 * u + rows * u, ea1w + u + rows * u
+    e_wt = (e_wsum_num + e_wsum_den) / 2 + 3 * u                         # division, sqrt, product with W: u each
+    e_norm = e_wt + DEPTH_F * u
+    e_vx1 = max(VX_IN_REL, e_wt + K * u) + u
+    e_a1h, e_a2h = e_vx1 + RCP_REL + (R - 1) * u, 2 * (e_vx1 + RCP_REL) + u + (R - 1) * u
+    e_hs = ((e_wt + e_a2h + 2 * u) + (e_wt + e_a1h + u)) / 2 + DEPTH_F * u + 3 * u
+    e_vb2 = e_wt + e_hs + K * u
+    e_vx2 = max(VX_IN_REL, e_vb2) + u
+    e_ng = 2 * (e_vx2 + RCP_REL) + 4 * u + (R + DEPTH_F) * u             # Vs / Vx (u), / Vx (u), E (u), P (u)
+    e_dg = e_vx2 + RCP_REL + 2 * u + (R + DEPTH_F) * u
+    e_g = (e_ng + e_dg) / 2 + 3 * u
+    e_vx3 = max(e_g + VX_IN_REL, e_vb2) + 3 * u                           # + the bin scale folded into g E and Vb
+    depth_c = 3 * R + DEPTH_F                                             # per-thread FP32 cost sum over <= 3 bins x R samples
+    pv = P / Vx3
+    per = (e_vx3 + QUAD_REL) * (1 + pv) + LG2_ABS * np.log(2.0) + depth_c * u * (1 + 2 * np.abs(np.log(Vx3)) + pv)
+    out.update(bound_W=(e_wt + e_norm + u) * out["W"], bound_H=(e_hs + e_norm + u) * out["H"], bound_g=e_g * gn,
+               bound_Vb=e_vb2 * Vb, bound_A1=e_a1 * A1, bound_A2=e_a2 * A2, rel_Wsum=(e_wsum_num, e_wsum_den),
+               bound_cost=per.mean() if per.size else 0.0)
+    vx = [Vx0, Vx1, Vx2, Vx3]
+    out["vx_min"] = min(float(v.min()) for v in vx) if Vs.size else 1.0
+    out["vx_max"] = max(float(v.max()) for v in vx) if Vs.size else 1.0
+    out["spread_log2"] = float(np.abs(np.log2(Vx3 / Vx3[:1])).max()) if Vs.size else 0.0
+    return out
+
+
+def m_step_in_range(ref):
+    """Whether the inputs of ``m_step_f64``'s result ``ref`` lie inside the range the M-step kernels handle (nmf.cu)."""
+    return VX_MIN <= ref["vx_min"] and ref["vx_max"] <= VX_MAX and ref["spread_log2"] <= BIN_SPREAD_LOG2
+
+
 def log_accept_reference(Vs_cur, Vs_prop, g, Vb, P, Z, Zp):
     """The log acceptance ratio of mcem.py:251-253 on explicit inputs ((F,N) variances, (L,N) latents)."""
     Vx, Vxp = g * Vs_cur + Vb, g * Vs_prop + Vb
