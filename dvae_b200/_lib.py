@@ -17,7 +17,7 @@ MAX_LAYERS = 6
 MAX_L = 64
 MAX_K = 16
 ACT_NONE, ACT_TANH, ACT_EXP = 0, 1, 2
-ABI_VERSION = 3
+ABI_VERSION = 4
 STATUS_TIMEOUT, STATUS_NONFINITE = 1, 2
 
 c_f32p = C.c_void_p      # device pointers are passed as integers
@@ -82,9 +82,8 @@ PROTOTYPES = {
                                   c_ptr, c_ptr]),
     "dvae_decode_stats_win_tc": (C.c_int, [C.POINTER(DvaeMlp), c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, C.c_int, c_ptr, C.c_int, c_ptr, c_ptr,
                                            c_ptr, C.c_int64, C.c_int, c_ptr, c_ptr, c_ptr, C.c_int, c_ptr, c_ptr]),
-    "dvae_decode_a1_tc": (C.c_int, [C.POINTER(DvaeMlp), c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, C.c_int, c_ptr, C.c_int, c_ptr, c_ptr, c_ptr,
-                                    C.c_int64, C.c_int, c_ptr, c_ptr, c_ptr]),
-    "dvae_wiener_from_a1": (C.c_int, [c_ptr, c_ptr, C.c_int, C.c_int64, C.c_int, C.c_int, c_ptr, c_ptr, C.c_int, c_ptr]),
+    "dvae_decode_wiener_tc": (C.c_int, [C.POINTER(DvaeMlp), c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, C.c_int, c_ptr, C.c_int, c_ptr, c_ptr,
+                                        c_ptr, C.c_int64, C.c_int, c_ptr, c_ptr, C.c_int, c_ptr, c_ptr]),
     "dvae_energy_ratios": (C.c_int, [c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, C.c_int, c_ptr, c_ptr]),
     "dvae_pcm16_f32": (C.c_int, [c_ptr, C.c_int64, c_ptr, c_ptr, c_ptr]),
     "dvae_resample_taps": (C.c_int, [C.c_int, c_ptr, C.c_int]),
@@ -97,6 +96,7 @@ PROTOTYPES = {
     "dvae_tc_decoder_exponent_bound": (C.c_int, [C.POINTER(DvaeMlp), C.c_int, C.c_int, c_ptr, c_ptr]),
     "dvae_tc_image_bias_offset": (C.c_int64, [C.POINTER(DvaeMlp), C.c_int, C.c_int]),
     "dvae_tc_tanh_bf16_table": (C.c_int, [c_ptr, c_ptr]),
+    "dvae_tc_tanh_f32": (C.c_int, [c_ptr, c_ptr, C.c_int64, c_ptr]),
     "dvae_decode_tc": (C.c_int, [C.POINTER(DvaeMlp), c_ptr, c_ptr, C.c_int64, C.c_int, c_ptr, C.c_int, c_ptr, C.c_int, c_ptr, C.c_int,
                                  c_ptr, c_ptr]),
     "dvae_vst_bytes": (C.c_int64, [C.c_int64, C.c_int]),

@@ -41,12 +41,14 @@ struct DsParams {
     const float* Vb;        // [NT][ld]
     const float* g;         // [NT]
     float* Vs;              // [NT][R][ld]
-    float* A1;              // [NT][ld]
-    float* A2;              // [NT][ld]
+    float* A1;              // [NT][ld] (STORE)
+    float* A2;              // [NT][ld] (STORE)
+    float* WFs;             // [NT][ld] (!STORE) mask sums sum_r g Vs / Vx ...
+    float* WFn;             // [NT][ld] (!STORE) ... and sum_r Vb / Vx
     int64_t NT;
     int ld;
     int zs_rtot, zs_r0;     // samples per frame in Zs (and Vs) and the first one this launch decodes (R of them)
-    int acc;                // != 0: add to A1 / A2 instead of overwriting (later sample windows of the same frames)
+    int acc;                // != 0: add to A1 / A2 (WFs / WFn) instead of overwriting (later sample windows of the same frames)
     int* status;
 };
 
@@ -89,8 +91,9 @@ __device__ __forceinline__ void ds_hidden_row(uint32_t tmem, unsigned char* A, i
 }
 
 // LDC: compile-time row pitch of Vs / Vb / A1 / A2 (520 for F = 513: store offsets become immediates), 0 = take p.ld
-// STORE = false: only A1 is produced (no Vs, no A2): the Wiener masks of the final filter follow from A1 alone,
-// mean_r g Vs / Vx = 1 - Vb A1 / R (mcem.py:325-327), so its 75 (25) samples are never written to memory.
+// STORE = false: the Wiener mask sums of the final filter (mcem.py:325-327) instead of Vs / A1 / A2, so its 75 (25) samples
+// are never written to memory: WFn = Vb sum_r 1 / Vx and WFs = g sum_r Vs / Vx.  The speech sum is accumulated, not taken
+// as R - Vb A1: where g Vs << Vb (collapsed gains, spectral nulls) that difference cancels to FP32 noise, even negative.
 template <int R, int L, int LDC, bool STORE>
 __global__ void __launch_bounds__(DS_THREADS, 1) decode_stats_kernel(DsParams p) {
     constexpr int RL = (R <= 16) ? 16 : 32;
@@ -266,8 +269,8 @@ __global__ void __launch_bounds__(DS_THREADS, 1) decode_stats_kernel(DsParams p)
                             // packed FP32 pairs; four samples share two reciprocals: X = (Vx_r, Vx_r+1), Y = (Vx_r+2, Vx_r+3),
                             // 1 / (X Y) gives 1 / X = Y / (X Y) and 1 / Y = X / (X Y) lane by lane
                             const f32x2 g2 = pk2(gg, gg), vb2 = pk2(vb, vb), bias2 = pk2(bias, bias);
-                            f32x2 a1p = 0ull, a2p = 0ull;
-                            float a1 = 0.f, a2 = 0.f;
+                            f32x2 a1p = 0ull, a2p = 0ull, asp = 0ull;
+                            float a1 = 0.f, a2 = 0.f, as = 0.f;          // as: sum_r Vs / Vx (STORE = false)
                             // CNT samples (rows r0 .. r0 + CNT of the frame) held in v[0 .. CNT)
                             auto quad = [&](const float* v, int k, int r0) {
                                 float e0, e1, e2, e3;
@@ -286,7 +289,8 @@ __global__ void __launch_bounds__(DS_THREADS, 1) decode_stats_kernel(DsParams p)
                                 const f32x2 rr = pk2(rcp_approx(m0), rcp_approx(m1));
                                 const f32x2 i0 = mul2(Y, rr), i1 = mul2(X, rr);
                                 a1p = add2(a1p, add2(i0, i1));
-                                a2p = fma2(i0, i0, fma2(i1, i1, a2p));
+                                if (STORE) a2p = fma2(i0, i0, fma2(i1, i1, a2p));
+                                else asp = fma2(pk2(s0, s1), i0, fma2(pk2(s2, s3), i1, asp));
                             };
                             auto pair = [&](const float* v, int k, int r0) {
                                 const float s0 = ex2_approx(v[k] + bias), s1 = ex2_approx(v[k + 1] + bias);
@@ -298,14 +302,16 @@ __global__ void __launch_bounds__(DS_THREADS, 1) decode_stats_kernel(DsParams p)
                                 const float rr = rcp_approx(x0 * x1);
                                 const float i0 = x1 * rr, i1 = x0 * rr;
                                 a1 += i0 + i1;
-                                a2 = fmaf(i0, i0, fmaf(i1, i1, a2));
+                                if (STORE) a2 = fmaf(i0, i0, fmaf(i1, i1, a2));
+                                else as = fmaf(s0, i0, fmaf(s1, i1, as));
                             };
                             auto single = [&](const float* v, int k, int r0) {
                                 const float s0 = ex2_approx(v[k] + bias);
                                 if (STORE) dst[(int64_t)(r0 + k) * ldv] = s0;
                                 const float i0 = rcp_approx(fmaf(gg, s0, vb));
                                 a1 += i0;
-                                a2 = fmaf(i0, i0, a2);
+                                if (STORE) a2 = fmaf(i0, i0, a2);
+                                else as = fmaf(s0, i0, as);
                             };
                             static_assert(R == 30 || R == 25 || R == 10, "sample count of the back epilogue");
                             float v0[16];
@@ -332,12 +338,25 @@ __global__ void __launch_bounds__(DS_THREADS, 1) decode_stats_kernel(DsParams p)
                                 float lo, hi;
                                 upk2(a1p, lo, hi);
                                 a1 += lo + hi;
-                                upk2(a2p, lo, hi);
-                                a2 += lo + hi;
+                                upk2(STORE ? a2p : asp, lo, hi);
+                                if (STORE) a2 += lo + hi;
+                                else as += lo + hi;
                             }
-                            if (p.acc) { a1 += p.A1[n * ldv + f]; if (STORE) a2 += p.A2[n * ldv + f]; }
-                            p.A1[n * ldv + f] = a1;
-                            if (STORE) p.A2[n * ldv + f] = a2;
+                            const int64_t i = n * ldv + f;
+                            bool finite;
+                            if (STORE) {
+                                if (p.acc) { a1 += p.A1[i]; a2 += p.A2[i]; }
+                                p.A1[i] = a1;
+                                p.A2[i] = a2;
+                                finite = isfinite(a1) && isfinite(a2);
+                            } else {
+                                float wn = __fmul_rn(vb, a1), ws = __fmul_rn(gg, as);   // no FMA contraction: WFn = fl(Vb A1)
+                                if (p.acc) { wn += p.WFn[i]; ws += p.WFs[i]; }
+                                p.WFn[i] = wn;
+                                p.WFs[i] = ws;
+                                finite = isfinite(wn) && isfinite(ws);
+                            }
+                            if (!finite) atomicOr(p.status, DVAE_STATUS_NONFINITE);
                         }
                     }
                 } else if (s == 0) {
@@ -348,14 +367,14 @@ __global__ void __launch_bounds__(DS_THREADS, 1) decode_stats_kernel(DsParams p)
                     float v[4];
                     tmem_ld4(tb + lane_off, v);
                     tmem_wait_ld();
-                    float inv = 0.f;
+                    float inv = 0.f, vs = 0.f;
                     if (fi < FT && n < p.NT && d.F > 512) {
-                        const float vs = ex2_approx(v[0] + b3[512]);
+                        vs = ex2_approx(v[0] + b3[512]);
                         if (STORE) p.Vs[(n * p.zs_rtot + p.zs_r0 + r) * (int64_t)ldv + 512] = vs;
                         inv = rcp_approx(fmaf(__ldg(p.g + n), vs, __ldg(p.Vb + n * ldv + 512)));
                     }
                     tailS[row] = inv;
-                    tailS[128 + row] = inv * inv;
+                    tailS[128 + row] = STORE ? inv * inv : vs * inv;
                     ds_bar_tail();
                     if (row < 2 * FT) {
                         const int fj = row >> 1, which = row & 1;
@@ -363,10 +382,16 @@ __global__ void __launch_bounds__(DS_THREADS, 1) decode_stats_kernel(DsParams p)
                         if (nn < p.NT && d.F > 512) {
                             float sum = 0.f;
                             for (int rr = 0; rr < R; ++rr) sum += tailS[which * 128 + fj * R + rr];
-                            if (STORE || which == 0) {
-                                float* dst512 = (which ? p.A2 : p.A1) + nn * ldv + 512;
-                                *dst512 = p.acc ? *dst512 + sum : sum;
+                            float* dst512;
+                            if (STORE) {
+                                dst512 = (which ? p.A2 : p.A1) + nn * ldv + 512;
+                            } else {
+                                dst512 = (which ? p.WFs : p.WFn) + nn * ldv + 512;
+                                sum = __fmul_rn(which ? __ldg(p.g + nn) : __ldg(p.Vb + nn * ldv + 512), sum);
                             }
+                            const float tot = p.acc ? *dst512 + sum : sum;
+                            *dst512 = tot;
+                            if (!isfinite(tot)) atomicOr(p.status, DVAE_STATUS_NONFINITE);
                         }
                     }
                     ds_bar_tail();
@@ -494,12 +519,12 @@ using namespace dvae::tc;
 
 static int launch_decode_stats(const char* who, const DvaeMlp* dec, const void* image, const float* Zs, int R_total, int r0, int R,
                                int L, const float* y, int y_dim, const float* ybias, const float* Vb, const float* g, int64_t NT, int ld, float* Vs,
-                               float* A1, float* A2, int accumulate, int* status, void* stream) {
+                               float* A1, float* A2, float* WFs, float* WFn, int accumulate, int* status, void* stream) {
     DsParams p{};
     int rc = check_dims(dec, L, y_dim, who, &p.d);
     if (rc) return rc;
     const bool store = Vs != nullptr;
-    DVAE_REQUIRE(image && Zs && Vb && g && A1 && status && (!store || A2), "%s: null pointer", who);
+    DVAE_REQUIRE(image && Zs && Vb && g && status && (store ? (A1 && A2) : (WFs && WFn)), "%s: null pointer", who);
     DVAE_REQUIRE(store ? (R == 10 || R == 30) : (R == 10 || R == 25 || R == 30), "%s: unsupported sample count %d", who, R);
     DVAE_REQUIRE(r0 >= 0 && r0 + R <= R_total, "%s: sample window [%d, %d) outside [0, %d)", who, r0, r0 + R, R_total);
     DVAE_REQUIRE(L == 16 || L == 32, "%s: latent size must be 16 or 32 (got %d)", who, L);
@@ -509,7 +534,7 @@ static int launch_decode_stats(const char* who, const DvaeMlp* dec, const void* 
                  "%s: Zs and image must be 16-byte aligned", who);
     if (NT == 0) return 0;
     p.image = (const unsigned char*)image;
-    p.Zs = Zs; p.y = y; p.ybias = ybias; p.Vb = Vb; p.g = g; p.Vs = Vs; p.A1 = A1; p.A2 = A2; p.NT = NT; p.ld = ld; p.status = status;
+    p.Zs = Zs; p.y = y; p.ybias = ybias; p.Vb = Vb; p.g = g; p.Vs = Vs; p.A1 = A1; p.A2 = A2; p.WFs = WFs; p.WFn = WFn; p.NT = NT; p.ld = ld; p.status = status;
     p.zs_rtot = R_total; p.zs_r0 = r0; p.acc = accumulate;
     const int shared_bytes = (p.d.off_w3 + 4 * ((p.d.n_hidden == 2 ? HID : 0) + NPAD) + 1023) & ~1023;
     const size_t smem = (size_t)shared_bytes + 65536 + (size_t)DS_NS * 32768 + 1024;
@@ -547,14 +572,15 @@ extern "C" int dvae_decode_stats_tc(const DvaeMlp* dec, const void* image, const
                                     int y_dim, const float* ybias, const float* Vb, const float* g, int64_t NT, int ld, float* Vs, float* A1,
                                     float* A2, int* status, void* stream) {
     DVAE_REQUIRE(Vs && A2, "dvae_decode_stats_tc: null pointer");
-    return launch_decode_stats("dvae_decode_stats_tc", dec, image, Zs, R, 0, R, L, y, y_dim, ybias, Vb, g, NT, ld, Vs, A1, A2, 0, status, stream);
+    return launch_decode_stats("dvae_decode_stats_tc", dec, image, Zs, R, 0, R, L, y, y_dim, ybias, Vb, g, NT, ld, Vs, A1, A2, nullptr, nullptr, 0,
+                               status, stream);
 }
 
-extern "C" int dvae_decode_a1_tc(const DvaeMlp* dec, const void* image, const float* Zs, int R_total, int r0, int R, int L,
-                                 const float* y, int y_dim, const float* ybias, const float* Vb, const float* g, int64_t NT, int ld, float* A1,
-                                 int* status, void* stream) {
-    return launch_decode_stats("dvae_decode_a1_tc", dec, image, Zs, R_total, r0, R, L, y, y_dim, ybias, Vb, g, NT, ld, nullptr, A1, nullptr,
-                               0, status, stream);
+extern "C" int dvae_decode_wiener_tc(const DvaeMlp* dec, const void* image, const float* Zs, int R_total, int r0, int R, int L,
+                                     const float* y, int y_dim, const float* ybias, const float* Vb, const float* g, int64_t NT, int ld,
+                                     float* WFs, float* WFn, int accumulate, int* status, void* stream) {
+    return launch_decode_stats("dvae_decode_wiener_tc", dec, image, Zs, R_total, r0, R, L, y, y_dim, ybias, Vb, g, NT, ld, nullptr, nullptr,
+                               nullptr, WFs, WFn, accumulate, status, stream);
 }
 
 // sample window [r0, r0 + R) of frames that hold R_total samples each (multi-chain runs): Vs rows n * R_total + r0 + r are
@@ -564,30 +590,7 @@ extern "C" int dvae_decode_stats_win_tc(const DvaeMlp* dec, const void* image, c
                                         float* A1, float* A2, int accumulate, int* status, void* stream) {
     DVAE_REQUIRE(Vs && A2, "dvae_decode_stats_win_tc: null pointer");
     return launch_decode_stats("dvae_decode_stats_win_tc", dec, image, Zs, R_total, r0, R, L, y, y_dim, ybias, Vb, g, NT, ld, Vs, A1, A2,
-                               accumulate, status, stream);
-}
-
-// WFn (+)= Vb A1, WFs (+)= R - Vb A1: sums over the R samples behind A1 of Vb / Vx and g Vs / Vx = 1 - Vb / Vx (mcem.py:325-327)
-__global__ void wiener_from_a1_kernel(const float* __restrict__ A1, const float* __restrict__ Vb, float R, int64_t NT, int F, int ld,
-                                      float* __restrict__ WFs, float* __restrict__ WFn, int first) {
-    const int64_t total = NT * ld;
-    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
-        const int f = (int)(i % ld);
-        if (f >= F) continue;
-        const float q = Vb[i] * A1[i];
-        WFn[i] = (first ? 0.f : WFn[i]) + q;
-        WFs[i] = (first ? 0.f : WFs[i]) + (R - q);
-    }
-}
-
-extern "C" int dvae_wiener_from_a1(const float* A1, const float* Vb, int R, int64_t NT, int F, int ld, float* WFs, float* WFn,
-                                   int first, void* stream) {
-    DVAE_REQUIRE(A1 && Vb && WFs && WFn && R >= 1 && NT >= 0 && F >= 1 && ld >= F, "dvae_wiener_from_a1: bad arguments");
-    if (NT == 0) return 0;
-    const int64_t blocks = (NT * ld + 255) / 256;
-    wiener_from_a1_kernel<<<(unsigned)(blocks < 148 * 16 ? blocks : 148 * 16), 256, 0, (cudaStream_t)stream>>>(A1, Vb, (float)R, NT, F, ld,
-                                                                                                            WFs, WFn, first);
-    return check_launch("wiener_from_a1_kernel");
+                               nullptr, nullptr, accumulate, status, stream);
 }
 
 extern "C" int dvae_nmf_w_from_frame_stats(const float* A1, const float* A2, const float* P, const float* H, const float* W,

@@ -473,6 +473,19 @@ extern "C" int dvae_tc_tanh_bf16_table(uint16_t* out, void* stream) {
     return check_launch("tanh_bf16_table_kernel");
 }
 
+// The decode kernels' hidden activation (hidden_epilogue_rows, ds_hidden_row): y[i] = tanh.approx.f32(x[i]); tests only
+__global__ void tanh_f32_kernel(const float* __restrict__ x, float* __restrict__ y, int64_t n) {
+    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) y[i] = tanh_approx(x[i]);
+}
+
+extern "C" int dvae_tc_tanh_f32(const float* x, float* y, int64_t n, void* stream) {
+    DVAE_REQUIRE(x && y && n >= 0, "dvae_tc_tanh_f32: bad arguments");
+    if (n == 0) return 0;
+    const int64_t blocks = (n + 255) / 256;
+    tanh_f32_kernel<<<(unsigned)(blocks < 148 * 32 ? blocks : 148 * 32), 256, 0, (cudaStream_t)stream>>>(x, y, n);
+    return check_launch("tanh_f32_kernel");
+}
+
 extern "C" int64_t dvae_tc_packed_pv_bytes(int64_t chains) {
     if (chains <= 0) return 0;
     return ((chains + TM - 1) / TM) * (int64_t)NQ * TM * 16;

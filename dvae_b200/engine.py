@@ -586,14 +586,11 @@ class McemEngine:
         WFs = self._get("WFs", (b.NT, self.ld))
         WFn = self._get("WFn", (b.NT, self.ld))
         if chunk:
-            # fused: the filter samples are decoded chunk by chunk straight into A1 = sum_r 1 / Vx; the masks follow from
-            # mean_r g Vs / Vx = 1 - Vb A1 / R, so none of the R x F x N variances is written to memory
+            # fused: the filter samples are decoded chunk by chunk straight into the mask sums, so none of the R x F x N
+            # variances is written to memory
             from . import tc
             for r0 in range(0, R, chunk):
-                A1 = tc.decode_a1_tc(self, Zs, r0, chunk)
-                _lib.call("dvae_wiener_from_a1", _p(A1), _p(self.Vb), chunk, b.NT, self.F, self.ld, _p(WFs), _p(WFn),
-                          1 if r0 == 0 else 0, _stream())
-                self.kernel_launches += 1
+                tc.decode_wiener_tc(self, Zs, r0, chunk, WFs, WFn, accumulate=r0 > 0)
         else:
             # decode in frame chunks so the Vs buffer of the E-step (NT * R_E rows) is reused
             flat = self.Vs_flat

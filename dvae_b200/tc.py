@@ -174,12 +174,11 @@ def decode_stats_tc(eng, Zs, Vs):
     return st
 
 
-def decode_a1_tc(eng, Zs, r0, R):
-    """A1 = sum over the samples r0 .. r0+R of 1 / (g Vs + Vb), without storing Vs (dvae_decode_a1_tc); ``[NT][ld]``."""
+def decode_wiener_tc(eng, Zs, r0, R, WFs, WFn, accumulate):
+    """Mask sums of the samples r0 .. r0+R of ``Zs`` without storing their variances (dvae_decode_wiener_tc):
+    ``WFs (+)= g sum_r Vs / Vx``, ``WFn (+)= Vb sum_r 1 / Vx``, ``[NT][ld]``."""
     w, b = eng.w, eng.batch
     img = decoder_image(w)
-    A1 = eng._get("wf_a1", (b.NT * eng.ld,))
-    _lib.call("dvae_decode_a1_tc", w.dec_tc.ref, _p(img), _p(Zs), Zs.shape[1], int(r0), int(R), w.z_dim, _p(eng.tc_y), w.tc_y_dim, _p(eng.ybias), _p(eng.Vb),
-              _p(eng.g), b.NT, eng.ld, _p(A1), _p(_status(eng)), _stream())
+    _lib.call("dvae_decode_wiener_tc", w.dec_tc.ref, _p(img), _p(Zs), Zs.shape[1], int(r0), int(R), w.z_dim, _p(eng.tc_y), w.tc_y_dim,
+              _p(eng.ybias), _p(eng.Vb), _p(eng.g), b.NT, eng.ld, _p(WFs), _p(WFn), int(bool(accumulate)), _p(_status(eng)), _stream())
     eng.kernel_launches += 1
-    return A1

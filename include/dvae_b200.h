@@ -31,7 +31,7 @@
 extern "C" {
 #endif
 
-#define DVAE_ABI_VERSION 3          /* 3: DvaeRng.iter0_frame appended */
+#define DVAE_ABI_VERSION 4          /* 4: dvae_decode_wiener_tc replaces dvae_decode_a1_tc + dvae_wiener_from_a1 */
 #define DVAE_ERR_ARG (-1)
 #define DVAE_MAX_LAYERS 6
 #define DVAE_MAX_L 64          /* latent dimension limit of the Metropolis-Hastings kernels */
@@ -213,6 +213,8 @@ int64_t dvae_tc_image_bias_offset(const DvaeMlp* dec, int L, int y_dim);
  * out[x] (65536 BF16 bit patterns, device memory) = the activation of the BF16 number with bit pattern x.  For parity tests:
  * the instruction is not the correctly rounded tanh. */
 int dvae_tc_tanh_bf16_table(uint16_t* out, void* stream);
+/* y[i] = tanh.approx.f32(x[i]), the activation of the decode kernels' hidden layers (tests: the float64 mirror's activation) */
+int dvae_tc_tanh_f32(const float* x, float* y, int64_t n, void* stream);
 int64_t dvae_vst_bytes(int64_t chains, int n_keep);
 int dvae_mh_chain_tc2(const DvaeMlp* dec, const void* image, const void* PVpk, const float* kscale, const float* g, const float* y, int y_dim,
                       const float* ybias /* nullable: [NT][128] */, const int32_t* frame_utt, const int32_t* frame_idx, float* Z,
@@ -264,13 +266,20 @@ int dvae_decode_stats_tc(const DvaeMlp* dec, const void* image, const float* Zs,
 int dvae_decode_stats_win_tc(const DvaeMlp* dec, const void* image, const float* Zs, int R_total, int r0, int R, int L,
                              const float* y, int y_dim, const float* ybias /* nullable */, const float* Vb, const float* g, int64_t NT, int ld, float* Vs, float* A1,
                              float* A2, int accumulate, int* status, void* stream);
-/* final filter without materialising its samples: dvae_decode_a1_tc decodes the samples r0 .. r0+R (R in {10, 25, 30}) of
- * every frame of Zs [NT][R_total][L] and writes only A1 = sum_r 1 / (g Vs + Vb); dvae_wiener_from_a1 then accumulates the
- * mask sums of compute_WF (mcem.py:325-327): sum_r Vb / Vx = Vb A1 and sum_r g Vs / Vx = R - Vb A1 (first != 0: overwrite) */
-int dvae_decode_a1_tc(const DvaeMlp* dec, const void* image, const float* Zs, int R_total, int r0, int R, int L, const float* y,
-                      int y_dim, const float* ybias /* nullable */, const float* Vb, const float* g, int64_t NT, int ld, float* A1, int* status, void* stream);
-int dvae_wiener_from_a1(const float* A1, const float* Vb, int R, int64_t NT, int F, int ld, float* WFs, float* WFn, int first,
-                        void* stream);
+/* Final filter without materialising its samples: dvae_decode_wiener_tc decodes the samples r0 .. r0+R (R in {10, 25, 30}) of
+ * every frame of Zs [NT][R_total][L] and writes the mask sums of compute_WF (mcem.py:325-327) for them, overwriting
+ * (accumulate == 0) or adding to WFs / WFn [NT][ld]:  WFs = g sum_r Vs / Vx,  WFn = Vb sum_r 1 / Vx.  Both sums are
+ * accumulated term by term (positive terms: FP32 relative precision in every bin, however small g Vs is against Vb).
+ * Supported range (this entry point, dvae_decode_stats_tc and dvae_decode_stats_win_tc; DESIGN section 6): every
+ * Vx = g Vs + Vb in [2^-60, 2^60], as for the M-step (the margin of 2^3 keeps A2 = sum_r Vx^-2 finite for R <= 256).
+ * Inside, Vs, A1 / A2 and the mask sums are within the error model of tests/test_gpu_decode_f64.py of float64.  Outside,
+ * the shared reciprocal of a pair of samples leaves FP32's normal range (at 2^-63 / 2^63): below, the pair product
+ * underflows, A1 / A2 / the mask sums become Inf or NaN and DVAE_STATUS_NONFINITE is OR-ed into *status; above, the pair
+ * product overflows, its reciprocal flushes to zero and those samples drop out of A1 / A2 / the sums: finite, too small,
+ * no status bit. */
+int dvae_decode_wiener_tc(const DvaeMlp* dec, const void* image, const float* Zs, int R_total, int r0, int R, int L, const float* y,
+                          int y_dim, const float* ybias /* nullable */, const float* Vb, const float* g, int64_t NT, int ld, float* WFs,
+                          float* WFn, int accumulate, int* status, void* stream);
 /* W <- W sqrt(num / den), num[f,k] = sum_n P A2 H, den[f,k] = sum_n A1 H (mcem.py:108-111); Wtmp: un-normalised result */
 int dvae_nmf_w_from_frame_stats(const float* A1, const float* A2, const float* P, const float* H, const float* W,
                                 const int64_t* fr_off, int B, int F, int K, int ld, float* Wtmp, void* stream);

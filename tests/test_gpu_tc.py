@@ -297,37 +297,6 @@ def test_multi_chain_emit_route_matches_stats_route(variant, keep, chains):
             assert err <= tol, "iteration %d: %s differs by %g" % (it, name, err)
 
 
-@pytest.mark.parametrize("R_total,chunk", [(75, 25), (30, 30), (25, 25), (20, 10)])
-def test_fused_wiener_a1_matches_materialised_samples(R_total, chunk):
-    """dvae_decode_a1_tc + dvae_wiener_from_a1 against the decode that writes Vs followed by dvae_wiener_accum."""
-    from dvae_b200 import tc as tcmod
-    N = [23, 9, 14]
-    rng = np.random.default_rng(4)
-    NT = sum(N)
-    P = torch.tensor(rng.gamma(1.0, 0.05, size=(NT, 520)).astype(np.float32)).to(DEV)
-    X = torch.zeros((NT, 520), dtype=torch.complex64, device=DEV)
-    sd = synth.xavier_state_dict("M1", 513, 16, [128, 128], 0, seed=3, out_bias=float(np.log(0.05)))
-    eng = McemEngine(VaeWeights(sd, "M1", DEV), McemConfig(niter=1, keep_E=30, burn_E=2, keep_WF=R_total, burn_WF=2, sampler="tc"), DEV)
-    eng.init_parameters(X, P, RaggedBatch(N, DEV))
-    eng.g.copy_(torch.tensor(rng.uniform(0.5, 2.0, size=NT).astype(np.float32)).to(DEV))
-    Zs = torch.tensor(rng.standard_normal((NT, R_total, 16)).astype(np.float32)).to(DEV)
-    WFs = torch.zeros((NT, 520), device=DEV)
-    WFn = torch.zeros((NT, 520), device=DEV)
-    for r0 in range(0, R_total, chunk):
-        A1 = tcmod.decode_a1_tc(eng, Zs, r0, chunk)
-        _lib.call("dvae_wiener_from_a1", _p(A1), _p(eng.Vb), chunk, NT, 513, 520, _p(WFs), _p(WFn), 1 if r0 == 0 else 0, _stream())
-    Vs = torch.empty((NT * R_total, 520), device=DEV)
-    eng.decode_samples(Zs, 0, NT, Vs)
-    Vs = Vs.view(NT, R_total, 520)[:, :, :513]
-    Vx = eng.g[:, None, None] * Vs + eng.Vb[:, None, :513]
-    ref_n = (eng.Vb[:, None, :513] / Vx).sum(1)
-    ref_s = (eng.g[:, None, None] * Vs / Vx).sum(1)
-    tcmod.check_status(eng)
-    assert float((WFn[:, :513] - ref_n).abs().max()) < 2e-4 * R_total
-    assert float((WFs[:, :513] - ref_s).abs().max()) < 2e-4 * R_total
-    assert float((WFs[:, :513] + WFn[:, :513] - R_total).abs().max()) < 1e-4 * R_total
-
-
 def test_sampler_handles_decoder_biases_spanning_many_decades():
     """A decoder whose output bias is tiny in part of the spectrum (a prior without energy above 3 kHz: exp(b3) ~ 1e-10 there)
     makes the sampler's bias-free variances X = Vx exp(-b3) huge in those bins.  With a fixed quad scale the four-fold products
