@@ -97,6 +97,7 @@ PROTOTYPES = {
     "dvae_tc_image_bias_offset": (C.c_int64, [C.POINTER(DvaeMlp), C.c_int, C.c_int]),
     "dvae_tc_tanh_bf16_table": (C.c_int, [c_ptr, c_ptr]),
     "dvae_tc_tanh_f32": (C.c_int, [c_ptr, c_ptr, C.c_int64, c_ptr]),
+    "dvae_box_muller_f32": (C.c_int, [c_ptr, c_ptr, c_ptr, c_ptr, C.c_int64, c_ptr]),
     "dvae_decode_tc": (C.c_int, [C.POINTER(DvaeMlp), c_ptr, c_ptr, C.c_int64, C.c_int, c_ptr, C.c_int, c_ptr, C.c_int, c_ptr, C.c_int,
                                  c_ptr, c_ptr]),
     "dvae_vst_bytes": (C.c_int64, [C.c_int64, C.c_int]),

@@ -98,7 +98,9 @@ __host__ __device__ __forceinline__ Philox4 philox4x32_10(uint32_t c0, uint32_t 
     return Philox4{c0, c1, c2, c3};
 }
 
-// (0,1) uniform from 24 random bits: never 0, never 1.
+// Uniform in (0, 1] from 24 random bits k: (k + 0.5) 2^-24 rounded to FP32.  Never 0.  For k >= 2^23 the sum k + 0.5 is a tie
+// between two FP32 neighbours and rounds to the even one, so the upper half sits on the 2^-23 grid and k = 2^24 - 1 gives
+// exactly 1.0 (one word in 2^24).  In box_muller, u1 = 1 gives a radius near 0 and u2 = 1 the angle fl(pi).
 __device__ __forceinline__ float u01(uint32_t r) { return ((float)(r >> 8) + 0.5f) * (1.0f / 16777216.0f); }
 
 // Box-Muller on two words -> two standard normals. Uses the MUFU approximations on purpose: the FP32 and the
@@ -114,7 +116,8 @@ __device__ __forceinline__ void box_muller(uint32_t a, uint32_t b, float& n0, fl
 
 // The accept uniform of an iteration: 24 bits collected from the LOW bytes of the first three words of Philox block 0.  The
 // normals of that block are built from the upper 24 bits of the same words (u01 / box_muller), so the uniform is independent of
-// them and costs no Philox evaluation of its own (inside the tensor-core sampler a block is ~150 instructions per chain).
+// them and costs no Philox evaluation of its own (inside the tensor-core sampler a block is ~150 instructions per chain).  Same
+// rounding as u01: in (0, 1], and exactly 1.0 when the 24 bits are all ones.
 __device__ __forceinline__ float u01_low_bytes(const Philox4& r) {
     const uint32_t v = (r.x & 255u) | ((r.y & 255u) << 8) | ((r.z & 255u) << 16);
     return ((float)v + 0.5f) * (1.0f / 16777216.0f);

@@ -306,6 +306,17 @@ __global__ void __launch_bounds__(256) rng_dump4_kernel(uint32_t seed_lo, uint32
     }
 }
 
+// box_muller on caller-supplied words; tests only (the float64 check of the normals over every 24-bit uniform)
+__global__ void box_muller_kernel(const uint32_t* __restrict__ a, const uint32_t* __restrict__ b, float* __restrict__ n0,
+                                  float* __restrict__ n1, int64_t n) {
+    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+        float x, y;
+        box_muller(a[i], b[i], x, y);
+        n0[i] = x;
+        n1[i] = y;
+    }
+}
+
 }  // namespace dvae
 
 using namespace dvae;
@@ -414,6 +425,7 @@ extern "C" int dvae_rng_dump(const DvaeRng* rng, const int32_t* frame_utt, const
                              int n_chains, int L, int n_iter, float* eps, float* u, void* stream) {
     DVAE_REQUIRE(rng && frame_utt && frame_idx && eps && u, "dvae_rng_dump: null pointer");
     DVAE_REQUIRE(NT >= 0 && n_chains >= 1 && L >= 1 && L <= DVAE_MAX_L && n_iter >= 0, "dvae_rng_dump: bad sizes");
+    DVAE_REQUIRE(n_chains < 4096, "dvae_rng_dump: n_chains=%d (the chain index has 12 bits of the counter)", n_chains);
     const int64_t total = NT * n_chains * n_iter;
     if (total == 0) return 0;
     if ((L == 4 || L == 8 || L == 16 || L == 32 || L == 64) && (reinterpret_cast<uintptr_t>(eps) & 15) == 0 && n_iter <= 65535 &&
@@ -433,4 +445,12 @@ extern "C" int dvae_rng_dump(const DvaeRng* rng, const int32_t* frame_utt, const
                                                            rng->iter0, rng->iter0_frame, frame_utt, frame_idx, NT * n_chains, n_chains, L,
                                                            n_iter, eps, u);
     return check_launch("rng_dump_kernel");
+}
+
+extern "C" int dvae_box_muller_f32(const uint32_t* a, const uint32_t* b, float* n0, float* n1, int64_t n, void* stream) {
+    DVAE_REQUIRE(a && b && n0 && n1 && n >= 0, "dvae_box_muller_f32: bad arguments");
+    if (n == 0) return 0;
+    const int64_t blocks = (n + 255) / 256;
+    box_muller_kernel<<<(unsigned)(blocks < 148 * 32 ? blocks : 148 * 32), 256, 0, (cudaStream_t)stream>>>(a, b, n0, n1, n);
+    return check_launch("box_muller_kernel");
 }

@@ -422,6 +422,7 @@ class McemEngine:
             raise ValueError("labels y are required exactly for the M2 variants")
         if y is not None and tuple(y.shape) != (batch.NT, w.y_dim):
             raise ValueError("y must be [NT][y_dim=%d]" % w.y_dim)
+        check_counters(batch.max_frames, cfg.n_chains)
         self.batch, self.X, self.P, self.y = batch, X, P, (None if y is None else y.contiguous().float())
         # what the tensor-core kernels see of the labels: the labels themselves (<= 3) or a per-frame layer-1 bias
         self.tc_y, self.ybias, self.kscale = self.y, None, None
@@ -782,6 +783,16 @@ def check_stop(cfg: McemConfig, draws=None, checkpoints: Sequence[int] = ()):
         raise ValueError("stop_tol needs the engine's own random numbers, not injected draws")
     if tuple(checkpoints):
         raise ValueError("stop_tol cannot be combined with score_at / checkpoints")
+
+
+def check_counters(max_frames: int, n_chains: int):
+    """``ValueError`` when two chains of a batch would draw the same random numbers.  Word 1 of a draw's Philox counter is
+    ``frame | chain << 20`` (csrc/common.cuh), so with several chains per frame an utterance of more than 2^20 frames (about
+    4.7 hours at the 256-sample hop of 16 kHz audio) would give frame 2^20 of chain 0 the counters of frame 0 of chain 1.
+    No device work."""
+    if n_chains > 1 and max_frames > 1 << 20:
+        raise ValueError("an utterance of %d frames exceeds the 2^20 frames per utterance that n_chains = %d leaves distinct "
+                         "random numbers for" % (max_frames, n_chains))
 
 
 def _bytes(t: torch.Tensor) -> torch.Tensor:

@@ -227,6 +227,8 @@ int64_t dvae_tc_image_bias_offset(const DvaeMlp* dec, int L, int y_dim);
 int dvae_tc_tanh_bf16_table(uint16_t* out, void* stream);
 /* y[i] = tanh.approx.f32(x[i]), the activation of the decode kernels' hidden layers (tests: the float64 mirror's activation) */
 int dvae_tc_tanh_f32(const float* x, float* y, int64_t n, void* stream);
+/* (n0[i], n1[i]) = the samplers' Box-Muller normals of the Philox words (a[i], b[i]) (csrc/common.cuh box_muller); tests only */
+int dvae_box_muller_f32(const uint32_t* a, const uint32_t* b, float* n0, float* n1, int64_t n, void* stream);
 int64_t dvae_vst_bytes(int64_t chains, int n_keep);
 int dvae_mh_chain_tc2(const DvaeMlp* dec, const void* image, const void* PVpk, const float* kscale, const float* g, const float* y, int y_dim,
                       const float* ybias /* nullable: [NT][128] */, const int32_t* frame_utt, const int32_t* frame_idx, float* Z,
