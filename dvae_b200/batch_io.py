@@ -113,7 +113,7 @@ def _read_checked(path, fs, length=None):
 
 
 def process_sublist(sublist, enhancer, processed_wav_dir, output_data_dir, batch_size=512, max_frames=None, labels=None,
-                    io_threads=8, fs=16000, utt_ids=None, score=False, score_at=()):
+                    io_threads=8, fs=16000, utt_ids=None, score=False, score_at=(), oracle_labels=None):
     """Batched replacement of ``process_sublist`` / ``process_utt`` (scripts/evaluate_ntcd_M1.py:81-214).
 
     ``sublist``: ``(proc_noisy_file_path, clean_file_path)`` pairs as the reference builds them.  Files whose
@@ -133,18 +133,30 @@ def process_sublist(sublist, enhancer, processed_wav_dir, output_data_dir, batch
     ``score_at`` (with ``score=True``): EM iteration counts as ``Enhancer.enhance(..., score_at=...)`` takes them; the call
     then returns ``(written_stems, scores, trace [n][len(score_at)][5])``, where ``trace[u][k]`` is the estimate's score row
     that a run with ``niter = score_at[k]`` would give, all from this one run.  The files do not change.
+
+    ``oracle_labels``: ``"vad"``, ``"ibm"`` or ``"robust_ibm"``, the M2 models' labels derived from the clean speech on the
+    device (``Enhancer.enhance(..., s_list=..., oracle_labels=...)``) instead of a ``labels`` callback.  The clean file of every
+    pair is read by the same read-ahead workers; with ``score=True`` that one read (and one upload) serves both the labels
+    and the scores.  Frame caps from ``max_frames`` cut the labels after they are computed on the whole clean signal.
     """
     score_at = tuple(score_at)
     if score_at and not score:
         raise ValueError("score_at needs score=True")
-    if score:
+    if oracle_labels is not None:
+        from .engine import ORACLE_LABELS
+        if oracle_labels not in ORACLE_LABELS:
+            raise ValueError("oracle_labels must be one of %s or None, got %r" % (ORACLE_LABELS, oracle_labels))
+        if labels is not None:
+            raise ValueError("oracle_labels and the labels callback are two sources of the same labels: pass one")
+    clean = score or oracle_labels is not None               # the clean file of every pair is read
+    if clean:
         _check_sublist(sublist, batch_size, fs, None)
     if score_at:
         from .engine import check_checkpoints
         score_at = check_checkpoints(score_at, enhancer.cfg.niter)
     utt_ids = utt_ids or utterance_id
     todo = [(a, b) for a, b in sublist if not os.path.exists(output_stem(output_data_dir, a) + "_s_est.wav")]
-    if score:
+    if clean:
         _require_files([processed_wav_dir + p for ab in todo for p in ab])
     written, scores, traces = [], [], []
     with ThreadPoolExecutor(max(1, io_threads)) as pool:
@@ -152,15 +164,15 @@ def process_sublist(sublist, enhancer, processed_wav_dir, output_data_dir, batch
 
         def submit_reads(part):
             return [(pool.submit(_read_checked, processed_wav_dir + ab[0], fs),
-                     pool.submit(_read_checked, processed_wav_dir + ab[1], fs) if score else None) for ab in part]
+                     pool.submit(_read_checked, processed_wav_dir + ab[1], fs) if clean else None) for ab in part]
 
         reads = submit_reads(todo[:batch_size])
         for lo in range(0, len(todo), batch_size):
             part = todo[lo:lo + batch_size]
             xs = [f.result() for f, _ in reads]
-            cs = [g.result() for _, g in reads] if score else None
+            cs = [g.result() for _, g in reads] if clean else None
             reads = submit_reads(todo[lo + batch_size:lo + 2 * batch_size])      # read ahead: the next batch loads while this one runs
-            if score:
+            if clean:
                 for x, c, ab in zip(xs, cs, part):
                     if len(c) != len(x):
                         raise ValueError("%s: %d samples, the noisy file has %d" % (processed_wav_dir + ab[1], len(c), len(x)))
@@ -170,13 +182,15 @@ def process_sublist(sublist, enhancer, processed_wav_dir, output_data_dir, batch
                 caps = [big if c is None else c for c in caps]
             ys = [labels(*ab) for ab in part] if labels else None
             ids = [utt_ids(ab[0]) for ab in part]
+            # the same list object for the labels and the scores: the enhancer then uploads the clean signals once
+            lab = {} if oracle_labels is None else dict(s_list=cs, oracle_labels=oracle_labels)
             if score:
                 s_hat, n_hat, _, sc, *tr = enhancer.enhance(xs, y_list=ys, max_frames_list=caps, utt_ids=ids, ref_list=cs, pcm16=True,
-                                                            score_at=score_at)
+                                                            score_at=score_at, **lab)
                 scores.append(sc)
                 traces += tr
             else:
-                s_hat, n_hat, _ = enhancer.enhance(xs, y_list=ys, max_frames_list=caps, utt_ids=ids)
+                s_hat, n_hat, _ = enhancer.enhance(xs, y_list=ys, max_frames_list=caps, utt_ids=ids, **lab)
             if pending:
                 for fut in pending:
                     fut.result()

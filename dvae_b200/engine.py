@@ -26,6 +26,7 @@ from . import _lib
 from .synth import FS, HOP, N_FFT, num_frames
 
 LD_ALIGN = 8
+ORACLE_LABELS = ("vad", "ibm", "robust_ibm")       # labels Enhancer.enhance derives from the clean speech (oracle_labels=)
 
 
 def _p(t: Optional[torch.Tensor]):
@@ -212,10 +213,14 @@ def _ld_for(F: int) -> int:
 
 
 def stft_batch(x_flat: torch.Tensor, x_off: torch.Tensor, x_len: torch.Tensor, batch: RaggedBatch, n_fft=N_FFT, hop=HOP,
-               want_power=True):
-    """STFT of a concatenated float32 device signal -> ``(X [NT][ld] complex64, P [NT][ld] float32 | None)``."""
-    ld = _ld_for(n_fft // 2 + 1)
-    X = torch.empty((batch.NT, ld), dtype=torch.complex64, device=x_flat.device)
+               want_power=True, ld=None, out=None):
+    """STFT of a concatenated float32 device signal -> ``(X [NT][ld] complex64, P [NT][ld] float32 | None)``.  ``ld``: row
+    stride in bins (default: ``n_fft / 2 + 1`` rounded up to a multiple of 8; at least ``n_fft / 2 + 1``); ``out``: a
+    contiguous complex64 ``[NT][ld]`` tensor to write ``X`` into."""
+    ld = _ld_for(n_fft // 2 + 1) if ld is None else int(ld)
+    if out is not None and (tuple(out.shape) != (batch.NT, ld) or out.dtype != torch.complex64 or not out.is_contiguous()):
+        raise ValueError("out must be a contiguous complex64 tensor [NT][ld=%d]" % ld)
+    X = out if out is not None else torch.empty((batch.NT, ld), dtype=torch.complex64, device=x_flat.device)
     P = torch.empty((batch.NT, ld), dtype=torch.float32, device=x_flat.device) if want_power else None
     with torch.cuda.device(x_flat.device):
         _lib.call("dvae_stft_f32", _p(x_flat), _p(x_off), _p(x_len), batch.B, _p(X), _p(P), _p(batch.fr_off), batch.NT,
@@ -927,17 +932,80 @@ class Enhancer:
             metrics.score_row(s_q, ref, rows[n])
         return score
 
+    def label_mode(self, oracle_labels, s_list, y_list):
+        """The oracle label mode of an ``enhance`` call (``ORACLE_LABELS`` or ``None``: labels from ``y_list`` or none);
+        ``ValueError`` when ``oracle_labels`` does not fit the model or the other arguments.  No device work."""
+        y_dim, F = self.weights.y_dim, self.n_fft // 2 + 1
+        if oracle_labels is None:
+            if not y_dim or y_list is not None or s_list is None:
+                return None
+            if y_dim != 1:
+                raise ValueError("a model with %d label inputs takes labels from s_list only with oracle_labels='ibm' or "
+                                 "'robust_ibm' (%d inputs)" % (y_dim, F))
+            return "vad"
+        if oracle_labels not in ORACLE_LABELS:
+            raise ValueError("oracle_labels must be one of %s or None, got %r" % (ORACLE_LABELS, oracle_labels))
+        if not y_dim:
+            raise ValueError("oracle_labels: an M1 model takes no labels")
+        if s_list is None:
+            raise ValueError("oracle_labels needs the clean signals s_list")
+        if y_list is not None:
+            raise ValueError("oracle_labels and y_list are two sources of the same labels: pass one")
+        want = 1 if oracle_labels == "vad" else F
+        if y_dim != want:
+            raise ValueError("oracle_labels=%r gives %d labels per frame, the model takes %d" % (oracle_labels, want, y_dim))
+        return oracle_labels
+
+    def oracle_labels_device(self, mode, s_dev, x_off, x_len, n_clean, batch):
+        """Oracle labels ``y [NT][y_dim]`` (engine buffers) of the clean signals ``s_dev`` (the layout of ``x_off`` / ``x_len``)
+        for the frames of ``batch``.  They are computed over all ``n_clean[u]`` frames of each clean signal - the VAD's
+        minimum frame power and the IBM's maximum magnitude are those of the whole utterance - and the first
+        ``batch.n_frames[u]`` frames are kept (one ``dvae_permute_rows`` gather when a cap cuts), which is how the reference
+        truncates ``y`` to the video length (scripts/evaluate_ntcd_M2.py:187-195).  The IBM's spectrogram and mask are laid
+        out with a row stride of ``F = n_fft / 2 + 1`` bins, so the mask is the dense label matrix itself.  Nothing
+        synchronises."""
+        from .packages.processing.target import ibm_batch, vad_batch
+        eng = self.engine
+        n_clean = np.asarray(n_clean, np.int64)
+        cut = bool(np.any(batch.n_frames != n_clean))
+        full = RaggedBatch(n_clean, self.dev) if cut else batch
+        NT = full.NT
+        vad = None
+        if mode in ("vad", "robust_ibm"):
+            vad = vad_batch(s_dev, x_off, x_len, full, self.n_fft, self.hop, out=eng._get("oracle_vad", (NT,)),
+                            ws=eng._get("oracle_vad_ws", (max(1, NT),), torch.float64))
+        if mode == "vad":
+            lab = vad.view(NT, 1)
+        else:
+            F = self.n_fft // 2 + 1
+            S, _ = stft_batch(s_dev, x_off, x_len, full, self.n_fft, self.hop, want_power=False, ld=F,
+                              out=eng._get("oracle_S", (NT, F), torch.complex64))
+            lab = ibm_batch(S, full, F, vad=vad, out=eng._get("oracle_ibm", (NT, F)),
+                            ws=eng._get("oracle_ibm_ws", (max(1, full.B),), torch.int32))
+        if not cut:
+            return lab
+        y = eng._get("oracle_y", (batch.NT, lab.shape[1]))
+        rows = np.repeat(full.fr_off_host[:-1] - batch.fr_off_host[:-1], batch.n_frames) + np.arange(batch.NT)
+        permute_rows([(lab, y, torch.from_numpy(rows.astype(np.int32)).to(self.dev), batch.NT, lab.shape[1] * 4, 1, 0)])
+        return y
+
     @_on_device
     def enhance(self, x_list, y_list=None, utt_ids=None, max_frames_list=None, draws=None, return_device=False, s_list=None,
-                ref_list=None, pcm16=False, score_at=()):
+                ref_list=None, pcm16=False, score_at=(), oracle_labels=None):
         """Enhance a list of 1-D float32 host signals.  Returns ``(s_hat_list, n_hat_list, cost [B][niter])``, and the scores
         ``[B][2][5]`` as a fourth element when ``ref_list`` is given, and the trace ``[B][len(score_at)][5]`` as a fifth when
         ``score_at`` is.
 
         ``y_list``: per-utterance label arrays ``(y_dim, N_u)`` as the reference passes them (M2 variants).
         ``max_frames_list``: optional per-utterance frame caps (the reference truncates to the video length).
-        ``s_list``: clean signals; for a model with one label input and no ``y_list`` the labels are the time-domain VAD
-        of the clean speech (``clean_speech_VAD``, scripts/evaluate_ntcd_M2.py), computed on the device.
+        ``s_list``: clean signals, one per utterance and of its length, from which the device computes the oracle labels of
+        scripts/evaluate_ntcd_M2.py (``oracle_labels_device``), so no label leaves or enters the host.
+        ``oracle_labels`` (with ``s_list``, not with ``y_list``): ``"vad"`` (``clean_speech_VAD``, one label input), ``"ibm"``
+        (``clean_speech_IBM`` of the clean STFT) or ``"robust_ibm"`` (``noise_robust_clean_speech_IBM``: the IBM times the
+        VAD), both for ``n_fft / 2 + 1`` label inputs.  ``None`` means ``"vad"`` for a model with one label input and
+        ``s_list``; a model with ``n_fft / 2 + 1`` label inputs needs the mode named.  Labels are computed over every frame of
+        the clean signal and then cut to the first ``min(N_u, cap_u)`` frames, as the reference cuts ``y`` to the video
+        length after computing it.
         ``utt_ids``: global utterance ids = Philox counter word 0; callers that enhance several batches must pass distinct
         ids per utterance (``batch_io.process_sublist`` does), or every batch replays the same random draws.
         ``ref_list``: clean signals, one per utterance and of its length, to score against on the device
@@ -968,6 +1036,10 @@ class Enhancer:
         score_at = check_checkpoints(score_at, eng.cfg.niter)
         if score_at and (ref_list is None or draws is not None):
             raise ValueError("score_at needs ref_list and the engine's own random numbers (no injected draws)")
+        mode = self.label_mode(oracle_labels, s_list, y_list)
+        if mode is not None and (len(s_list) != B or any(len(a) != t for a, t in zip(s_list, lens))):
+            raise ValueError("oracle labels need one clean signal per utterance, of the utterance's length")
+        nfr_clean = nfr                            # the frames the oracle labels are computed over (truncation rule)
         if max_frames_list is not None:
             nfr = np.minimum(nfr, np.asarray(max_frames_list, np.int64))
         off = np.zeros(B + 1, np.int64)
@@ -982,14 +1054,12 @@ class Enhancer:
         x_len = torch.from_numpy(lens).to(dev)
         batch = RaggedBatch(nfr, dev, utt_ids)
         y = s_dev_in = None
-        if self.weights.y_dim and y_list is None and s_list is not None:
-            if self.weights.y_dim != 1 or len(s_list) != B or any(len(a) != t for a, t in zip(s_list, lens)):
-                raise ValueError("device VAD labels need one clean signal per utterance and a model with one label input")
-            from .packages.processing.target import vad_batch
+        y_up = 0                                   # label bytes copied from the host
+        if mode is not None:
             hs_in = self._pin("s_in", total, torch.float32)
             self._stage(hs_in.numpy(), s_list, off, lens)
             s_dev_in = hs_in.to(dev, non_blocking=True)
-            y = vad_batch(s_dev_in, x_off, x_len, batch, self.n_fft, self.hop).view(batch.NT, 1)
+            y = self.oracle_labels_device(mode, s_dev_in, x_off, x_len, nfr_clean, batch)
         elif self.weights.y_dim:
             if y_list is None:
                 raise ValueError("this model needs labels y")
@@ -997,6 +1067,7 @@ class Enhancer:
             if yc.shape != (batch.NT, self.weights.y_dim):
                 raise ValueError("labels do not cover the frames")
             y = torch.from_numpy(np.ascontiguousarray(yc)).to(dev)
+            y_up = y.numel() * 4
         ref_dev = None
         if ref_list is not None:
             if ref_list is s_list and s_dev_in is not None:
@@ -1015,7 +1086,8 @@ class Enhancer:
                                                    batch, total, int(lens.max()), {n: trace[:, k] for k, n in enumerate(score_at)})
         side = tuple(n for n in score_at if n < eng.cfg.niter)    # niter itself is the run's own filter, scored below
         s_dev, n_dev, cost = self.run_device(x_dev, x_off, x_len, batch, y, total, int(lens.max()), draws, side, on_checkpoint)
-        self.h2d_bytes = total * 4 + (0 if y is None else y.numel() * 4) + (0 if ref_dev is None else total * 4)
+        clean_up = (s_dev_in is not None) + (ref_dev is not None and ref_dev is not s_dev_in)    # clean signals uploaded
+        self.h2d_bytes = total * 4 * (1 + clean_up) + y_up
         scores = None
         if ref_list is not None or pcm16:
             from .packages import metrics

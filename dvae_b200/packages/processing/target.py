@@ -15,21 +15,32 @@ from ...engine import RaggedBatch, _ld_for, _p, _stream
 from ...synth import num_frames
 
 
-def vad_batch(x_flat, x_off, x_len, batch: RaggedBatch, n_fft=1024, hop=256, vad_threshold=1.70):
-    """``[NT]`` float32 labels for a concatenated float32 device signal (frames of ``RaggedBatch``)."""
-    vad = torch.empty(batch.NT, dtype=torch.float32, device=x_flat.device)
-    ws = torch.empty(max(1, batch.NT), dtype=torch.float64, device=x_flat.device)
+def _buffer(t, shape, dtype, device, what):
+    if t is None:
+        return torch.empty(shape, dtype=dtype, device=device)
+    if t.dtype != dtype or not t.is_contiguous() or t.numel() < int(np.prod(shape)):
+        raise ValueError("%s must be a contiguous %s tensor of at least %d elements" % (what, dtype, int(np.prod(shape))))
+    return t
+
+
+def vad_batch(x_flat, x_off, x_len, batch: RaggedBatch, n_fft=1024, hop=256, vad_threshold=1.70, out=None, ws=None):
+    """``[NT]`` float32 labels for a concatenated float32 device signal (frames of ``RaggedBatch``).  ``out`` (float32,
+    ``NT`` elements) and ``ws`` (float64, ``max(1, NT)`` elements): caller-owned buffers, allocated when not given."""
+    vad = _buffer(out, (batch.NT,), torch.float32, x_flat.device, "out")[:batch.NT]
+    ws = _buffer(ws, (max(1, batch.NT),), torch.float64, x_flat.device, "ws")
     with torch.cuda.device(x_flat.device):
         _lib.call("dvae_vad_labels", _p(x_flat), _p(x_off), _p(x_len), batch.B, _p(batch.frame_utt), _p(batch.fr_off), batch.NT,
                   n_fft, hop, float(vad_threshold), _p(vad), _p(ws), _stream())
     return vad
 
 
-def ibm_batch(S, batch: RaggedBatch, F, eps=1e-8, ibm_threshold=50, vad=None):
-    """``[NT][ld]`` float32 mask of a frame-major complex64 spectrogram ``S [NT][ld]`` (optionally gated by ``vad [NT]``)."""
+def ibm_batch(S, batch: RaggedBatch, F, eps=1e-8, ibm_threshold=50, vad=None, out=None, ws=None):
+    """``[NT][ld]`` float32 mask of a frame-major complex64 spectrogram ``S [NT][ld]`` (optionally gated by ``vad [NT]``).
+    ``out`` (float32 ``[NT][ld]``) and ``ws`` (int32, ``max(1, B)`` elements): caller-owned buffers, allocated when not
+    given.  With ``ld = F`` the mask is the dense ``[NT][F]`` label matrix the M2 models read."""
     ld = S.shape[1]
-    mask = torch.empty((batch.NT, ld), dtype=torch.float32, device=S.device)
-    ws = torch.empty(max(1, batch.B), dtype=torch.int32, device=S.device)
+    mask = _buffer(out, (batch.NT, ld), torch.float32, S.device, "out").view(-1)[:batch.NT * ld].view(batch.NT, ld)
+    ws = _buffer(ws, (max(1, batch.B),), torch.int32, S.device, "ws")
     with torch.cuda.device(S.device):
         _lib.call("dvae_ibm_labels", _p(S), _p(batch.frame_utt), _p(batch.fr_off), batch.B, batch.NT, F, ld, float(eps),
                   float(ibm_threshold), _p(vad), _p(mask), _p(ws), _stream())
